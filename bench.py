@@ -4,6 +4,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
   python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU solver, all host cores
+  python bench.py ... --dump-outputs DIR                   # also write the last timed step's results to DIR/*.npy
 
 A "step" is what icoFoam does per pressure solve: the assembled coefficients go into the
 solver's layout (b200ldu_matrix_set = the reference's calcSortCoeffs, lduMatrix.C:380-471) and
@@ -428,6 +429,7 @@ def main():
     ap.add_argument("--no-parity", action="store_true", help="skip the parity gate (profiling runs only)")
     ap.add_argument("--no-secondary", action="store_true", help="skip the PBiCG / GAMG / channel-like legs")
     ap.add_argument("--with-context", action="store_true", help="reference arm: also time the port and stock DIC")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
 
@@ -513,6 +515,8 @@ def main():
     ev1.record()
     barrier()
     ms = max_over_ranks(ev0.elapsed_time(ev1))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, psi.cpu().numpy(), perf, rank, world)
     launches = ctx.launches - l0
     value = nGlobal * iters * args.steps / (ms * 1e-3) / 1e6
     # the solve alone (round-1 definition of the step), for the roofline of the iteration kernels
@@ -654,6 +658,21 @@ def main():
         dist.destroy_process_group()
 
 
+def dump_outputs(path, psi, perf, rank, world):
+    """What the last timed step hands its caller, as float64 .npy files: the solution psi and its solver performance.
+    psi is a fixed, seeded sample of 2^21 cells over all ranks where it is larger (psi_cells.npy: which cells, in the
+    rank's numbering), so that the files stay within 32 MB and two builds can be compared value for value."""
+    os.makedirs(path, exist_ok=True)
+    sfx = f".rank{rank}" if world > 1 else ""
+    cap = (1 << 21) // world
+    cells = np.arange(len(psi)) if len(psi) <= cap else np.sort(np.random.default_rng(0).choice(len(psi), cap, replace=False))
+    np.save(os.path.join(path, f"psi{sfx}.npy"), psi[cells].astype(np.float64))
+    np.save(os.path.join(path, f"psi_cells{sfx}.npy"), cells.astype(np.float64))
+    np.save(os.path.join(path, f"solver_performance{sfx}.npy"),
+            np.array([perf.initialResidual, perf.finalResidual, perf.normFactor, perf.nIterations, perf.converged,
+                      perf.singular], np.float64))
+
+
 def sum_faces(meshmod, n, world):
     """internal faces held by all ranks together (the coefficients every rank uploads in the e2e arm)"""
     nx, ny, nz = meshmod.brick_split(world)
@@ -669,7 +688,7 @@ def secondary_legs(args, capi, torch, dist, meshmod, ctx, addr, mesh, dev, rank,
     out = {}
     tt = lambda a: torch.from_numpy(np.ascontiguousarray(a)).to(dev)
     N, F = mesh.nCells, mesh.nFaces
-    steps = max(2, min(args.steps, 3))
+    steps = args.steps
 
     def timed(fn):
         for _ in range(2):

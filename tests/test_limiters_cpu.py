@@ -6,8 +6,11 @@ import ctypes as C
 import numpy as np
 import pytest
 
+import ref_replay
 from oracle import limiters_oracle as lo
 from test_host_kernels_cpu import hk  # noqa: F401  (fixture: the host build of the kernels)
+
+ref_replay.install()   # the reference's answers come from tests/golden/ref_calls_*.npz
 
 
 def _case(meshmod, dims=(9, 7, 5), seed=3):
@@ -23,7 +26,6 @@ def _case(meshmod, dims=(9, 7, 5), seed=3):
     return m, vf, gradc, flux, cd, m.cell_centres()
 
 
-@pytest.mark.skipif(not lo.reference_available(), reason="oracle/_ref/libref_limiters.so not built")
 @pytest.mark.parametrize("scheme,k", [("limitedLinear", 1.0), ("limitedLinear", 0.33), ("limitedLinear", 0.0), ("vanLeer", 1.0),
                                       ("Minmod", 1.0)])
 def test_oracle_limiters_match_the_reference_headers(meshmod, scheme, k):

@@ -8,8 +8,11 @@ import importlib
 import numpy as np
 import pytest
 
+import ref_replay
 from oracle import mules_oracle as mo
 from test_host_kernels_cpu import Host, _d, hk  # noqa: F401  (fixture: the host build of the kernels)
+
+ref_replay.install()   # the reference's answers come from tests/golden/ref_calls_*.npz
 
 COMBOS = ["one-zero", "rho", "SpSu", "rho-SpSu"]
 
@@ -44,7 +47,6 @@ def _cat(a, b):
     return np.concatenate([a, b])
 
 
-@pytest.mark.skipif(not mo.reference_available(), reason="oracle/_ref/libref_mules.so not built")
 @pytest.mark.parametrize("combo", COMBOS)
 @pytest.mark.parametrize("nIter", [0, 1, 3])
 def test_oracle_matches_the_reference_mules(meshmod, combo, nIter):
@@ -69,7 +71,6 @@ def test_oracle_matches_the_reference_mules(meshmod, combo, nIter):
     assert np.array_equal(new, ref)
 
 
-@pytest.mark.skipif(not mo.reference_available(), reason="oracle/_ref/libref_mules.so not built")
 def test_oracle_matches_the_reference_other_bounds(meshmod):
     """psiMax / psiMin that cut into the field (the local extrema are clipped to them)"""
     d = case(meshmod, (5, 6, 3), seed=9)
@@ -202,7 +203,6 @@ def decomposed_fluxes(meshmod, dims, nRanks, rank, seed=5):
     return decomposed(meshmod, dims, nRanks, seed)[4][rank].mules_fluxes
 
 
-@pytest.mark.skipif(not mo.reference_available(), reason="oracle/_ref/libref_mules.so not built")
 @pytest.mark.parametrize("nRanks,combo", [(2, "one-zero"), (4, "rho-SpSu"), (8, "SpSu")])
 def test_oracle_matches_the_reference_on_a_decomposed_case(meshmod, nRanks, combo):
     """processor patches: psi of the neighbour cells in the extrema, the coupled face rule, the minimum with the other side"""
@@ -280,7 +280,6 @@ def corr_case(meshmod, dims, seed, combo):
     return d
 
 
-@pytest.mark.skipif(not mo.reference_available(), reason="oracle/_ref/libref_mules.so not built")
 @pytest.mark.parametrize("combo", COMBOS)
 @pytest.mark.parametrize("extremaCoeff", [0.0, 0.1])
 def test_oracle_matches_the_reference_cmules(meshmod, combo, extremaCoeff):

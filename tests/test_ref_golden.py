@@ -30,9 +30,9 @@ def _oracle(meshmod, orc, dims, kind):
 
 
 def test_fixture_is_reproducible_where_the_reference_is_present(meshmod, ref_golden):
+    import ref_replay
     from oracle import ref_ldu
-    if not ref_ldu.available():
-        pytest.skip("oracle/_ref not built and /root/reference absent")
+    ref_replay.install()   # the reference's answers come from tests/golden/ref_calls_*.npz
     fresh = mrg.generate(meshmod, ref_ldu)
     assert sorted(fresh) == sorted(ref_golden.files)
     for k in ref_golden.files:

@@ -12,10 +12,10 @@ import importlib
 import numpy as np
 import pytest
 
+import ref_replay
 from oracle import ref_ldu
 
-pytestmark = pytest.mark.skipif(not ref_ldu.available(),
-                                reason="oracle/_ref not built and /root/reference absent")
+ref_replay.install()   # the reference's answers come from tests/golden/ref_calls_*.npz
 
 
 def _pair(meshmod, orc, dims, kind):
@@ -560,15 +560,26 @@ def test_merged_coarse_interfaces_match_reference_code(meshmod, orc):
         assert np.array_equal(flat, o["patchFaceRestrict"])
         assert np.array_equal(g["faceCells"], o["faceCells"])
 
-from hypothesis import given, settings, strategies as st  # noqa: E402
+
+def _random_examples(n=30, seed=20240611):
+    """(dims, seed, symmetric, favourSpeed) of the property below: the smallest and largest boxes, then seeded draws --
+    the same examples on every run, so that the reference's answers for them can be stored"""
+    rng = np.random.default_rng(seed)
+    out = [((1, 1, 1), 0, True, 0), ((6, 6, 5), 1, False, 2)]
+    while len(out) < n:
+        dims = (int(rng.integers(1, 7)), int(rng.integers(1, 7)), int(rng.integers(1, 6)))
+        out.append((dims, int(rng.integers(0, 2**31)), bool(rng.integers(0, 2)), int(rng.integers(0, 3))))
+    return out
 
 
-@settings(max_examples=30, deadline=None)
-@given(st.tuples(st.integers(1, 6), st.integers(1, 6), st.integers(1, 5)), st.integers(0, 2**31 - 1), st.booleans(),
-       st.sampled_from([0, 1, 2]))
-def test_random_matrices_match_reference_code(dims, seed, symmetric, favourSpeed):
+def test_random_matrices_match_reference_code():
     """property: on any hex box with arbitrary coefficients the oracle's row operations equal the
     reference's code bit for bit (any favourSpeed path)"""
+    for dims, seed, symmetric, favourSpeed in _random_examples():
+        _random_matrix_matches_reference_code(dims, seed, symmetric, favourSpeed)
+
+
+def _random_matrix_matches_reference_code(dims, seed, symmetric, favourSpeed):
     import importlib as _il
     meshmod = _il.import_module("rapidcfd-dev_b200.mesh")
     from oracle import ldu_oracle as orc
