@@ -9,7 +9,7 @@
 // (src/Pstream/mpi/allReduceTemplates.C:197).
 //
 // Peer-memory path (default when CUDA IPC works; B200LDU_P2P=0 forces NCCL):
-//  * every rank cudaMalloc's one small region and publishes its IPC handle (all-gathered
+//  * every rank allocates one small device region and publishes its IPC handle (all-gathered
 //    with NCCL at b200ldu_comm_init); every rank maps every other region;
 //  * halo: the pack kernel gathers psi at the patch face cells and stores it STRAIGHT INTO
 //    THE NEIGHBOUR'S receive buffer over NVLink (coalesced peer stores), then releases a
@@ -55,12 +55,12 @@ static int p2p_setup(b200ldu_ctx *ctx)
     if (ctx->nRanks > P2P_MAXR) return B200LDU_OK;
     cudaStream_t st = ctx->stream;
     ncclComm_t comm = (ncclComm_t)ctx->nccl;
-    CUDA_TRY(cudaMalloc((void **)&ctx->region, P2P_REGION_BYTES));
-    CUDA_TRY(cudaMemsetAsync(ctx->region, 0, P2P_REGION_BYTES, st));
-    CUDA_TRY(cudaMalloc((void **)&ctx->d_seq, 64 * sizeof(unsigned long long)));
-    CUDA_TRY(cudaMemsetAsync(ctx->d_seq, 0, 64 * sizeof(unsigned long long), st));
+    TRY(ctx->region.alloc(P2P_REGION_BYTES));
+    CUDA_TRY(cudaMemsetAsync(ctx->region.get(), 0, P2P_REGION_BYTES, st));
+    TRY(ctx->d_seq.alloc(64));
+    CUDA_TRY(cudaMemsetAsync(ctx->d_seq.get(), 0, 64 * sizeof(unsigned long long), st));
     cudaIpcMemHandle_t mine;
-    cudaError_t ce = cudaIpcGetMemHandle(&mine, ctx->region);
+    cudaError_t ce = cudaIpcGetMemHandle(&mine, ctx->region.get());
     int ok = (ce == cudaSuccess) ? 1 : 0;
     if (!ok) cudaGetLastError();
     // all-gather {ok, handle} through NCCL (device buffers)
@@ -69,15 +69,15 @@ static int p2p_setup(b200ldu_ctx *ctx)
     memcpy(sendH.data(), &ok, sizeof(int));
     memcpy(sendH.data() + 64, &mine, sizeof(mine));
     static_assert(sizeof(cudaIpcMemHandle_t) == 64, "IPC handle is 64 bytes");
-    char *d_send = nullptr, *d_all = nullptr;
-    CUDA_TRY(cudaMalloc((void **)&d_send, rec));
-    CUDA_TRY(cudaMalloc((void **)&d_all, (size_t)rec * ctx->nRanks));
-    CUDA_TRY(cudaMemcpyAsync(d_send, sendH.data(), rec, cudaMemcpyHostToDevice, st));
-    NCCL_TRY(ncclAllGather(d_send, d_all, rec, ncclChar, comm, st));
-    CUDA_TRY(cudaMemcpyAsync(allH.data(), d_all, (size_t)rec * ctx->nRanks, cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(cudaStreamSynchronize(st));
-    cudaFree(d_send);
-    cudaFree(d_all);
+    {
+        DevBuf<char> d_send, d_all;
+        TRY(d_send.alloc(rec));
+        TRY(d_all.alloc((size_t)rec * ctx->nRanks));
+        CUDA_TRY(cudaMemcpyAsync(d_send.get(), sendH.data(), rec, cudaMemcpyHostToDevice, st));
+        NCCL_TRY(ncclAllGather(d_send.get(), d_all.get(), rec, ncclChar, comm, st));
+        CUDA_TRY(cudaMemcpyAsync(allH.data(), d_all.get(), (size_t)rec * ctx->nRanks, cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaStreamSynchronize(st));
+    }
     bool all = true;
     for (int r = 0; r < ctx->nRanks; r++) {
         int okr;
@@ -88,7 +88,7 @@ static int p2p_setup(b200ldu_ctx *ctx)
     if (all) {
         for (int r = 0; r < ctx->nRanks && opened; r++) {
             if (r == ctx->rank) {
-                ctx->peerRegion[r] = ctx->region;
+                ctx->peerRegion[r] = ctx->region.get();
                 continue;
             }
             cudaIpcMemHandle_t h;
@@ -103,13 +103,12 @@ static int p2p_setup(b200ldu_ctx *ctx)
         }
     }
     // every rank must agree (a rank that failed to map falls everybody back to NCCL)
-    int *d_flag = nullptr;
-    CUDA_TRY(cudaMalloc((void **)&d_flag, sizeof(int)));
-    CUDA_TRY(cudaMemcpyAsync(d_flag, &opened, sizeof(int), cudaMemcpyHostToDevice, st));
-    NCCL_TRY(ncclAllReduce(d_flag, d_flag, 1, ncclInt, ncclMin, comm, st));
-    CUDA_TRY(cudaMemcpyAsync(&opened, d_flag, sizeof(int), cudaMemcpyDeviceToHost, st));
+    DevBuf<int> d_flag;
+    TRY(d_flag.alloc(1));
+    CUDA_TRY(cudaMemcpyAsync(d_flag.get(), &opened, sizeof(int), cudaMemcpyHostToDevice, st));
+    NCCL_TRY(ncclAllReduce(d_flag.get(), d_flag.get(), 1, ncclInt, ncclMin, comm, st));
+    CUDA_TRY(cudaMemcpyAsync(&opened, d_flag.get(), sizeof(int), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
-    cudaFree(d_flag);
     ctx->p2p = opened != 0;
     return B200LDU_OK;
 }
@@ -144,14 +143,12 @@ extern "C" int b200ldu_comm_info(const b200ldu_ctx *ctx, const b200ldu_addr *a, 
 
 int comm_destroy(b200ldu_ctx *ctx)
 {
-    if (ctx->region) {
+    // the peers' regions are unmapped before this rank's own is released
+    if (ctx->region.get())
         for (int r = 0; r < ctx->nRanks; r++)
             if (r != ctx->rank && ctx->peerRegion[r]) cudaIpcCloseMemHandle(ctx->peerRegion[r]);
-        cudaFree(ctx->region);
-        ctx->region = nullptr;
-    }
-    if (ctx->d_seq) cudaFree(ctx->d_seq);
-    ctx->d_seq = nullptr;
+    ctx->region.reset();
+    ctx->d_seq.reset();
     if (ctx->nccl) {
         ncclCommDestroy((ncclComm_t)ctx->nccl);
         ctx->nccl = nullptr;
@@ -175,7 +172,7 @@ P2PRed comm_p2p_red(b200ldu_ctx *ctx)
         p.mail[r] = (double *)(ctx->peerRegion[r] + P2P_MAIL_OFF);
         p.flag[r] = (unsigned long long *)(ctx->peerRegion[r] + P2P_MAILFLAG_OFF);
     }
-    p.seq = ctx->d_seq; // [0]
+    p.seq = ctx->d_seq.get(); // [0]
     return p;
 }
 
@@ -213,15 +210,15 @@ int comm_addr_setup(b200ldu_addr *a)
     if (!simple)
         for (int r = 0; r < R; r++) row[r] = -2;
     row[2 * R] = a->nCells;
-    int *d_row = nullptr, *d_all = nullptr;
-    CUDA_TRY(cudaMalloc((void **)&d_row, sizeof(int) * row.size()));
-    CUDA_TRY(cudaMalloc((void **)&d_all, sizeof(int) * all.size()));
-    CUDA_TRY(cudaMemcpyAsync(d_row, row.data(), sizeof(int) * row.size(), cudaMemcpyHostToDevice, st));
-    NCCL_TRY(ncclAllGather(d_row, d_all, row.size(), ncclInt, comm, st));
-    CUDA_TRY(cudaMemcpyAsync(all.data(), d_all, sizeof(int) * all.size(), cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(cudaStreamSynchronize(st));
-    cudaFree(d_row);
-    cudaFree(d_all);
+    {
+        DevBuf<int> d_row, d_all;
+        TRY(d_row.alloc(row.size()));
+        TRY(d_all.alloc(all.size()));
+        CUDA_TRY(cudaMemcpyAsync(d_row.get(), row.data(), sizeof(int) * row.size(), cudaMemcpyHostToDevice, st));
+        NCCL_TRY(ncclAllGather(d_row.get(), d_all.get(), row.size(), ncclInt, comm, st));
+        CUDA_TRY(cudaMemcpyAsync(all.data(), d_all.get(), sizeof(int) * all.size(), cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaStreamSynchronize(st));
+    }
     double ncg = 0;
     bool everySimple = true;
     for (int r = 0; r < R; r++) {
@@ -253,23 +250,19 @@ int comm_addr_setup(b200ldu_addr *a)
             pc.push_back({p, a->patchStart[p] + c * PACK_CHUNK, std::min(a->patchStart[p] + (c + 1) * PACK_CHUNK, a->patchStart[p + 1])});
         a->L.nbr[a->L.nNbr++] = nb;
     }
-    PackPatch *d_pp = nullptr;
-    PackChunk *d_pc = nullptr;
-    CUDA_TRY(cudaMalloc((void **)&d_pp, sizeof(PackPatch) * pp.size()));
-    CUDA_TRY(cudaMalloc((void **)&d_pc, sizeof(PackChunk) * pc.size()));
-    CUDA_TRY(cudaMemcpy(d_pp, pp.data(), sizeof(PackPatch) * pp.size(), cudaMemcpyHostToDevice));
-    CUDA_TRY(cudaMemcpy(d_pc, pc.data(), sizeof(PackChunk) * pc.size(), cudaMemcpyHostToDevice));
-    a->d_packPatches = d_pp;
-    a->d_packChunks = d_pc;
+    TRY(a->d_packPatches.alloc(pp.size()));
+    TRY(a->d_packChunks.alloc(pc.size()));
+    CUDA_TRY(cudaMemcpy(a->d_packPatches.get(), pp.data(), sizeof(PackPatch) * pp.size(), cudaMemcpyHostToDevice));
+    CUDA_TRY(cudaMemcpy(a->d_packChunks.get(), pc.data(), sizeof(PackChunk) * pc.size(), cudaMemcpyHostToDevice));
     a->nPackChunks = (int)pc.size();
-    a->L.haloFlags = (const unsigned long long *)(ctx->region + P2P_HALOFLAG_OFF);
-    a->L.haloSeq = ctx->d_seq + 1;
-    a->L.tail0 = (const double *)(ctx->region + P2P_RECV_OFF);
+    a->L.haloFlags = (const unsigned long long *)(ctx->region.get() + P2P_HALOFLAG_OFF);
+    a->L.haloSeq = ctx->d_seq.get() + 1;
+    a->L.tail0 = (const double *)(ctx->region.get() + P2P_RECV_OFF);
     a->L.tail1 = a->L.tail0 + P2P_RECV_CAP;
-    a->L.packChunks = d_pc;
-    a->L.packPatches = d_pp;
-    a->L.sendRows = a->d_sendRows;
-    a->L.seqs = ctx->d_seq;
+    a->L.packChunks = a->d_packChunks.get();
+    a->L.packPatches = a->d_packPatches.get();
+    a->L.sendRows = a->d_sendRows.get();
+    a->L.seqs = ctx->d_seq.get();
     a->L.nPackChunks = (int)pc.size();
     a->p2pHalo = true;
     return B200LDU_OK;
@@ -308,13 +301,13 @@ int comm_halo_exchange(b200ldu_addr *a, double *x, double *sendBuf, const int *s
     bool remote = false;
     for (int p = 0; p < a->nPatches; p++)
         if (a->neighbRank[p] >= 0) remote = true;
-    if (a->d_cyclicSrc) { // cyclic partners: x[nPad + face] = x[partner's face cell]
-        cyclic_fill_kernel<<<(nRecv + 255) / 256, 256, 0, ctx->stream>>>(nRecv, a->d_cyclicSrc, x, x + a->L.nPad, stop);
+    if (a->d_cyclicSrc.get()) { // cyclic partners: x[nPad + face] = x[partner's face cell]
+        cyclic_fill_kernel<<<(nRecv + 255) / 256, 256, 0, ctx->stream>>>(nRecv, a->d_cyclicSrc.get(), x, x + a->L.nPad, stop);
         ctx->launches++;
         KERNEL_CHECK();
     }
     if (!remote) return B200LDU_OK;
-    pack_kernel<<<(nRecv + 255) / 256, 256, 0, ctx->stream>>>(nRecv, a->d_sendRows, x, sendBuf, stop);
+    pack_kernel<<<(nRecv + 255) / 256, 256, 0, ctx->stream>>>(nRecv, a->d_sendRows.get(), x, sendBuf, stop);
     ctx->launches++;
     KERNEL_CHECK();
     if (remote && !ctx->nccl) {
@@ -365,27 +358,25 @@ int comm_exchange_patch_ints(b200ldu_ctx *ctx, int nPatches, const int *patchSta
         b200_set_error("processor patches present but no communicator (b200ldu_comm_init)");
         return B200LDU_ENCCL;
     }
-    int *d_s = nullptr, *d_r = nullptr;
-    CUDA_TRY(cudaMalloc((void **)&d_s, sizeof(int) * (size_t)tot));
-    CUDA_TRY(cudaMalloc((void **)&d_r, sizeof(int) * (size_t)tot));
+    DevBuf<int> d_s, d_r;
+    TRY(d_s.alloc((size_t)tot));
+    TRY(d_r.alloc((size_t)tot));
     cudaStream_t st = ctx->stream;
-    CUDA_TRY(cudaMemcpyAsync(d_s, send, sizeof(int) * (size_t)tot, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(d_s.get(), send, sizeof(int) * (size_t)tot, cudaMemcpyHostToDevice, st));
     NCCL_TRY(ncclGroupStart());
     for (int p = 0; p < nPatches; p++) {
         int s = patchStart[p], n = patchStart[p + 1] - s;
         if (neighbRank[p] < 0) continue;
-        NCCL_TRY(ncclSend(d_s + s, n, ncclInt, neighbRank[p], (ncclComm_t)ctx->nccl, st));
-        NCCL_TRY(ncclRecv(d_r + s, n, ncclInt, neighbRank[p], (ncclComm_t)ctx->nccl, st));
+        NCCL_TRY(ncclSend(d_s.get() + s, n, ncclInt, neighbRank[p], (ncclComm_t)ctx->nccl, st));
+        NCCL_TRY(ncclRecv(d_r.get() + s, n, ncclInt, neighbRank[p], (ncclComm_t)ctx->nccl, st));
     }
     NCCL_TRY(ncclGroupEnd());
     std::vector<int> got((size_t)tot);
-    CUDA_TRY(cudaMemcpyAsync(got.data(), d_r, sizeof(int) * (size_t)tot, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(got.data(), d_r.get(), sizeof(int) * (size_t)tot, cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     for (int p = 0; p < nPatches; p++)
         if (neighbRank[p] >= 0)
             for (int i = patchStart[p]; i < patchStart[p + 1]; i++) recv[i] = got[i];
-    cudaFree(d_s);
-    cudaFree(d_r);
     return B200LDU_OK;
 }
 
@@ -396,16 +387,14 @@ int comm_allgather_host(b200ldu_ctx *ctx, const double *mine, int n, double *all
         memcpy(all, mine, sizeof(double) * (size_t)n);
         return B200LDU_OK;
     }
-    double *d_s = nullptr, *d_a = nullptr;
+    DevBuf<double> d_s, d_a;
     cudaStream_t st = ctx->stream;
-    CUDA_TRY(cudaMalloc((void **)&d_s, sizeof(double) * (size_t)n));
-    CUDA_TRY(cudaMalloc((void **)&d_a, sizeof(double) * (size_t)n * ctx->nRanks));
-    CUDA_TRY(cudaMemcpyAsync(d_s, mine, sizeof(double) * (size_t)n, cudaMemcpyHostToDevice, st));
-    NCCL_TRY(ncclAllGather(d_s, d_a, n, ncclDouble, (ncclComm_t)ctx->nccl, st));
-    CUDA_TRY(cudaMemcpyAsync(all, d_a, sizeof(double) * (size_t)n * ctx->nRanks, cudaMemcpyDeviceToHost, st));
+    TRY(d_s.alloc((size_t)n));
+    TRY(d_a.alloc((size_t)n * ctx->nRanks));
+    CUDA_TRY(cudaMemcpyAsync(d_s.get(), mine, sizeof(double) * (size_t)n, cudaMemcpyHostToDevice, st));
+    NCCL_TRY(ncclAllGather(d_s.get(), d_a.get(), n, ncclDouble, (ncclComm_t)ctx->nccl, st));
+    CUDA_TRY(cudaMemcpyAsync(all, d_a.get(), sizeof(double) * (size_t)n * ctx->nRanks, cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
-    cudaFree(d_s);
-    cudaFree(d_a);
     return B200LDU_OK;
 }
 

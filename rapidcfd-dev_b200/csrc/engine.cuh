@@ -264,5 +264,5 @@ int engine_launch(b200ldu_addr *a, const double *val, const Op &op)
 template <class Op>
 int engine_launch_m(b200ldu_matrix *m, bool transpose, const Op &op)
 {
-    return engine_launch(m->a, transpose ? m->d_valT : m->d_val, op);
+    return engine_launch(m->a, transpose ? m->valT() : m->d_val.get(), op);
 }

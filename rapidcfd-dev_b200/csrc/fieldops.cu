@@ -81,7 +81,7 @@ extern "C" int b200ldu_fv_sngrad(b200ldu_addr *a, int nComp, const double *delta
     if (a->nFaces == 0) return B200LDU_OK;
     CUDA_TRY(cudaSetDevice(a->ctx->device));
     const long long tot = (long long)a->nFaces * nComp;
-    sngrad_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, a->ctx->stream>>>(a->nFaces, nComp, a->d_l, a->d_u, deltaCoeffs_d, vf_d,
+    sngrad_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, a->ctx->stream>>>(a->nFaces, nComp, a->d_l.get(), a->d_u.get(), deltaCoeffs_d, vf_d,
                                                                              out_d);
     a->ctx->launches++;
     KERNEL_CHECK();
@@ -118,7 +118,7 @@ extern "C" int b200ldu_fv_limiter(b200ldu_addr *a, const char *scheme, double k,
     if (a->nFaces == 0) return B200LDU_OK;
     CUDA_TRY(cudaSetDevice(a->ctx->device));
     const double kk = k > 1e-15 ? k : 1e-15;   // twoByk_ = 2.0/max(k_, SMALL), SMALL = 1e-15 (doubleScalar.H)
-    limiter_kernel<<<(a->nFaces + 255) / 256, 256, 0, a->ctx->stream>>>(a->nFaces, sch, 2.0 / kk, a->d_l, a->d_u, faceFlux_d, vf_d,
+    limiter_kernel<<<(a->nFaces + 255) / 256, 256, 0, a->ctx->stream>>>(a->nFaces, sch, 2.0 / kk, a->d_l.get(), a->d_u.get(), faceFlux_d, vf_d,
                                                                        gradc_d, C_d, limiter_d);
     a->ctx->launches++;
     KERNEL_CHECK();

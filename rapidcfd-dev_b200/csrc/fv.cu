@@ -39,14 +39,9 @@ extern "C" int b200ldu_fv_boundary_set(b200ldu_addr *a, int nBFaces, const int *
         for (int i = 0; i < nBFaces; i++) faces[cur[bFaceCells_h[i]]++] = i;
     }
     std::vector<int> fc(bFaceCells_h, bFaceCells_h + nBFaces);
-    for (int **p : {&a->d_bFaceCells, &a->d_bCellStart, &a->d_bCellFaces})
-        if (*p) {
-            cudaFree(*p);
-            *p = nullptr;
-        }
-    TRY(dev_upload(&a->d_bFaceCells, fc));
-    TRY(dev_upload(&a->d_bCellStart, start));
-    TRY(dev_upload(&a->d_bCellFaces, faces));
+    TRY(a->d_bFaceCells.upload(fc));
+    TRY(a->d_bCellStart.upload(start));
+    TRY(a->d_bCellFaces.upload(faces));
     a->nBFaces = nBFaces;
     return B200LDU_OK;
 }
@@ -58,15 +53,15 @@ extern "C" int b200ldu_fv_surface_integrate(b200ldu_addr *a, int nComp, const do
     if (!a || !ssf_d || !out_d || (divideByV && !V_d) || (nComp != 1 && nComp != 3)) return B200LDU_EINVAL;
     if (a->nBFaces && !bssf_d) return B200LDU_EINVAL;
     CUDA_TRY(cudaSetDevice(a->ctx->device));
-    const int *bs = a->nBFaces ? a->d_bCellStart : nullptr;
+    const int *bs = a->nBFaces ? a->d_bCellStart.get() : nullptr;
     dim3 g((a->nCells + 127) / 128), b(128);
     if (nComp == 1)
-        surface_integrate_kernel<1><<<g, b, 0, a->ctx->stream>>>(a->nCells, a->d_ownerStart, a->d_losortStart,
-                                                                  a->d_losort, bs, a->d_bCellFaces, ssf_d, bssf_d,
+        surface_integrate_kernel<1><<<g, b, 0, a->ctx->stream>>>(a->nCells, a->d_ownerStart.get(), a->d_losortStart.get(),
+                                                                  a->d_losort.get(), bs, a->d_bCellFaces.get(), ssf_d, bssf_d,
                                                                   V_d, out_d, divideByV, neiSign);
     else
-        surface_integrate_kernel<3><<<g, b, 0, a->ctx->stream>>>(a->nCells, a->d_ownerStart, a->d_losortStart,
-                                                                  a->d_losort, bs, a->d_bCellFaces, ssf_d, bssf_d,
+        surface_integrate_kernel<3><<<g, b, 0, a->ctx->stream>>>(a->nCells, a->d_ownerStart.get(), a->d_losortStart.get(),
+                                                                  a->d_losort.get(), bs, a->d_bCellFaces.get(), ssf_d, bssf_d,
                                                                   V_d, out_d, divideByV, neiSign);
     a->ctx->launches++;
     KERNEL_CHECK();
@@ -80,15 +75,15 @@ extern "C" int b200ldu_fv_gauss_grad(b200ldu_addr *a, int nComp, const double *S
     if (!a || !Sf_d || !ssf_d || !V_d || !out_d || (nComp != 1 && nComp != 3)) return B200LDU_EINVAL;
     if (a->nBFaces && (!bSf_d || !bssf_d)) return B200LDU_EINVAL;
     CUDA_TRY(cudaSetDevice(a->ctx->device));
-    const int *bs = a->nBFaces ? a->d_bCellStart : nullptr;
+    const int *bs = a->nBFaces ? a->d_bCellStart.get() : nullptr;
     dim3 g((a->nCells + 127) / 128), b(128);
     if (nComp == 1)
-        gauss_grad_kernel<1><<<g, b, 0, a->ctx->stream>>>(a->nCells, a->d_ownerStart, a->d_losortStart,
-                                                           a->d_losort, bs, a->d_bCellFaces, Sf_d, ssf_d, bSf_d,
+        gauss_grad_kernel<1><<<g, b, 0, a->ctx->stream>>>(a->nCells, a->d_ownerStart.get(), a->d_losortStart.get(),
+                                                           a->d_losort.get(), bs, a->d_bCellFaces.get(), Sf_d, ssf_d, bSf_d,
                                                            bssf_d, V_d, out_d);
     else
-        gauss_grad_kernel<3><<<g, b, 0, a->ctx->stream>>>(a->nCells, a->d_ownerStart, a->d_losortStart,
-                                                           a->d_losort, bs, a->d_bCellFaces, Sf_d, ssf_d, bSf_d,
+        gauss_grad_kernel<3><<<g, b, 0, a->ctx->stream>>>(a->nCells, a->d_ownerStart.get(), a->d_losortStart.get(),
+                                                           a->d_losort.get(), bs, a->d_bCellFaces.get(), Sf_d, ssf_d, bSf_d,
                                                            bssf_d, V_d, out_d);
     a->ctx->launches++;
     KERNEL_CHECK();
@@ -123,8 +118,8 @@ extern "C" int b200ldu_fv_laplacian_fill(b200ldu_addr *a, const double *deltaCoe
     CUDA_TRY(cudaSetDevice(a->ctx->device));
     cudaStream_t st = a->ctx->stream;
     if (a->nFaces) laplacian_upper_kernel<<<(a->nFaces + 255) / 256, 256, 0, st>>>(a->nFaces, deltaCoeffs_d, gammaMagSf_d, upper_d);
-    neg_sum_diag_kernel<<<(a->nCells + 127) / 128, 128, 0, st>>>(a->nCells, a->d_ownerStart, a->d_losortStart,
-                                                                  a->d_losort, upper_d, upper_d, diag_d);
+    neg_sum_diag_kernel<<<(a->nCells + 127) / 128, 128, 0, st>>>(a->nCells, a->d_ownerStart.get(), a->d_losortStart.get(),
+                                                                  a->d_losort.get(), upper_d, upper_d, diag_d);
     a->ctx->launches += 2;
     KERNEL_CHECK();
     return B200LDU_OK;
@@ -137,8 +132,8 @@ extern "C" int b200ldu_fv_convection_fill(b200ldu_addr *a, const double *weights
     CUDA_TRY(cudaSetDevice(a->ctx->device));
     cudaStream_t st = a->ctx->stream;
     if (a->nFaces) convection_faces_kernel<<<(a->nFaces + 255) / 256, 256, 0, st>>>(a->nFaces, weights_d, phi_d, lower_d, upper_d);
-    neg_sum_diag_kernel<<<(a->nCells + 127) / 128, 128, 0, st>>>(a->nCells, a->d_ownerStart, a->d_losortStart,
-                                                                  a->d_losort, upper_d, lower_d, diag_d);
+    neg_sum_diag_kernel<<<(a->nCells + 127) / 128, 128, 0, st>>>(a->nCells, a->d_ownerStart.get(), a->d_losortStart.get(),
+                                                                  a->d_losort.get(), upper_d, lower_d, diag_d);
     a->ctx->launches += 2;
     KERNEL_CHECK();
     return B200LDU_OK;
@@ -166,9 +161,9 @@ extern "C" int b200ldu_fv_interpolate_linear(b200ldu_addr *a, int nComp, const d
     if (a->nFaces == 0) return B200LDU_OK;
     dim3 g((a->nFaces + 255) / 256), b(256);
     if (nComp == 1)
-        interpolate_linear_kernel<1><<<g, b, 0, a->ctx->stream>>>(a->nFaces, a->d_l, a->d_u, w_d, vf_d, sf_d);
+        interpolate_linear_kernel<1><<<g, b, 0, a->ctx->stream>>>(a->nFaces, a->d_l.get(), a->d_u.get(), w_d, vf_d, sf_d);
     else
-        interpolate_linear_kernel<3><<<g, b, 0, a->ctx->stream>>>(a->nFaces, a->d_l, a->d_u, w_d, vf_d, sf_d);
+        interpolate_linear_kernel<3><<<g, b, 0, a->ctx->stream>>>(a->nFaces, a->d_l.get(), a->d_u.get(), w_d, vf_d, sf_d);
     a->ctx->launches++;
     KERNEL_CHECK();
     return B200LDU_OK;
@@ -192,8 +187,8 @@ static int add_boundary(b200ldu_addr *a, const double *coeffs, double *x)
     if (!a || !coeffs || !x) return B200LDU_EINVAL;
     if (!a->nBFaces) return B200LDU_OK;
     CUDA_TRY(cudaSetDevice(a->ctx->device));
-    add_boundary_kernel<<<(a->nCells + 255) / 256, 256, 0, a->ctx->stream>>>(a->nCells, a->d_bCellStart,
-                                                                             a->d_bCellFaces, coeffs, x);
+    add_boundary_kernel<<<(a->nCells + 255) / 256, 256, 0, a->ctx->stream>>>(a->nCells, a->d_bCellStart.get(),
+                                                                             a->d_bCellFaces.get(), coeffs, x);
     a->ctx->launches++;
     KERNEL_CHECK();
     return B200LDU_OK;
@@ -221,15 +216,15 @@ extern "C" int b200ldu_fv_grad_linear(b200ldu_addr *a, int nComp, const double *
     if (!a || !Sf_d || !w_d || !vf_d || !V_d || !out_d || (nComp != 1 && nComp != 3)) return B200LDU_EINVAL;
     if (a->nBFaces && (!bSf_d || !bvf_d)) return B200LDU_EINVAL;
     CUDA_TRY(cudaSetDevice(a->ctx->device));
-    const int *bs = a->nBFaces ? a->d_bCellStart : nullptr;
+    const int *bs = a->nBFaces ? a->d_bCellStart.get() : nullptr;
     dim3 g((a->nCells + 127) / 128), b(128);
     if (nComp == 1)
-        grad_linear_kernel<1><<<g, b, 0, a->ctx->stream>>>(a->nCells, a->d_ownerStart, a->d_u, a->d_losortStart,
-                                                            a->d_losort, a->d_l, bs, a->d_bCellFaces, Sf_d, w_d, vf_d,
+        grad_linear_kernel<1><<<g, b, 0, a->ctx->stream>>>(a->nCells, a->d_ownerStart.get(), a->d_u.get(), a->d_losortStart.get(),
+                                                            a->d_losort.get(), a->d_l.get(), bs, a->d_bCellFaces.get(), Sf_d, w_d, vf_d,
                                                             bSf_d, bvf_d, V_d, out_d);
     else
-        grad_linear_kernel<3><<<g, b, 0, a->ctx->stream>>>(a->nCells, a->d_ownerStart, a->d_u, a->d_losortStart,
-                                                            a->d_losort, a->d_l, bs, a->d_bCellFaces, Sf_d, w_d, vf_d,
+        grad_linear_kernel<3><<<g, b, 0, a->ctx->stream>>>(a->nCells, a->d_ownerStart.get(), a->d_u.get(), a->d_losortStart.get(),
+                                                            a->d_losort.get(), a->d_l.get(), bs, a->d_bCellFaces.get(), Sf_d, w_d, vf_d,
                                                             bSf_d, bvf_d, V_d, out_d);
     a->ctx->launches++;
     KERNEL_CHECK();
@@ -262,7 +257,7 @@ extern "C" int b200ldu_fv_flux_linear(b200ldu_addr *a, const double *Sf_d, const
     if (!a || !Sf_d || !w_d || !U_d || !phi_d) return B200LDU_EINVAL;
     CUDA_TRY(cudaSetDevice(a->ctx->device));
     if (a->nFaces == 0) return B200LDU_OK;
-    flux_linear_kernel<<<(a->nFaces + 255) / 256, 256, 0, a->ctx->stream>>>(a->nFaces, a->d_l, a->d_u, Sf_d, w_d, U_d,
+    flux_linear_kernel<<<(a->nFaces + 255) / 256, 256, 0, a->ctx->stream>>>(a->nFaces, a->d_l.get(), a->d_u.get(), Sf_d, w_d, U_d,
                                                                              phi_d);
     a->ctx->launches++;
     KERNEL_CHECK();

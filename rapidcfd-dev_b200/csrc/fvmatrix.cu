@@ -15,8 +15,6 @@
 // element-wise field algebra around it (the /V, the +source, the max / divide / subtract of relax) is fused
 // into the same pass.  Products are rounded separately and summed in the reference's order, so the results
 // are bit-comparable with the oracle.
-#include <algorithm>
-
 #include "comm.h"
 #include "fieldops_kernels.cuh"
 #include "fvmatrix_kernels.cuh"
@@ -29,7 +27,7 @@ namespace
 {
 int coupled_lists(b200ldu_addr *a)
 {
-    if (a->d_cCellStart || a->nPatches == 0) return B200LDU_OK;
+    if (a->d_cCellStart.get() || a->nPatches == 0) return B200LDU_OK;
     const int tot = a->patchStart.empty() ? 0 : a->patchStart[a->nPatches];
     if (tot == 0) return B200LDU_OK;
     std::vector<int> start((size_t)a->nCells + 1, 0), faces((size_t)tot);
@@ -37,9 +35,9 @@ int coupled_lists(b200ldu_addr *a)
     for (int c = 0; c < a->nCells; c++) start[c + 1] += start[c];
     std::vector<int> cur(start.begin(), start.end() - 1);
     for (int i = 0; i < tot; i++) faces[cur[a->faceCells[i]]++] = i;
-    TRY(dev_upload(&a->d_cCellStart, start));
-    TRY(dev_upload(&a->d_cCellFaces, faces));
-    TRY(dev_upload(&a->d_cFaceCells, a->faceCells));
+    TRY(a->d_cCellStart.upload(start));
+    TRY(a->d_cCellFaces.upload(faces));
+    TRY(a->d_cFaceCells.upload(a->faceCells));
     a->nCFaces = tot;
     return B200LDU_OK;
 }
@@ -47,22 +45,10 @@ int coupled_lists(b200ldu_addr *a)
 int lists(b200ldu_addr *a, BoundaryLists *L)
 {
     TRY(coupled_lists(a));
-    L->bStart = a->nBFaces ? a->d_bCellStart : nullptr;
-    L->bFaces = a->d_bCellFaces;
-    L->cStart = a->nCFaces ? a->d_cCellStart : nullptr;
-    L->cFaces = a->d_cCellFaces;
-    return B200LDU_OK;
-}
-
-int scratch(b200ldu_addr *a, int slot, size_t doubles, double **out)
-{
-    if (a->fvmScratchLen[slot] < doubles) {
-        if (a->d_fvmScratch[slot]) CUDA_TRY(cudaFree(a->d_fvmScratch[slot]));
-        a->d_fvmScratch[slot] = nullptr;
-        CUDA_TRY(cudaMalloc((void **)&a->d_fvmScratch[slot], sizeof(double) * std::max<size_t>(doubles, 1)));
-        a->fvmScratchLen[slot] = doubles;
-    }
-    *out = a->d_fvmScratch[slot];
+    L->bStart = a->nBFaces ? a->d_bCellStart.get() : nullptr;
+    L->bFaces = a->d_bCellFaces.get();
+    L->cStart = a->nCFaces ? a->d_cCellStart.get() : nullptr;
+    L->cFaces = a->d_cCellFaces.get();
     return B200LDU_OK;
 }
 
@@ -89,13 +75,13 @@ extern "C" int b200ldu_fv_patch_neighbour_field(b200ldu_addr *a, int nComp, cons
     TRY(coupled_lists(a));
     if (a->nCFaces == 0) return B200LDU_OK;
     if (!pnf_d) return B200LDU_EINVAL;
-    double *send = nullptr;
-    TRY(scratch(a, 3, (size_t)a->nCFaces * nComp, &send));
-    fieldk::gather_kernel<<<grid(a->nCFaces * nComp, 256), 256, 0, a->ctx->stream>>>(a->nCFaces, nComp, a->d_cFaceCells,
-                                                                                      field_d, send);
+    DevBuf<double> &send = a->fvmScratch[FVM_CMPT_PSI];
+    TRY(send.grow((size_t)a->nCFaces * nComp));
+    fieldk::gather_kernel<<<grid(a->nCFaces * nComp, 256), 256, 0, a->ctx->stream>>>(a->nCFaces, nComp, a->d_cFaceCells.get(),
+                                                                                      field_d, send.get());
     a->ctx->launches++;
     KERNEL_CHECK();
-    return comm_exchange_patch_field(a, nComp, send, pnf_d);
+    return comm_exchange_patch_field(a, nComp, send.get(), pnf_d);
 }
 
 extern "C" int b200ldu_fvm_add_boundary_diag(b200ldu_matrix *m, int nComp, int cmpt, const double *internalCoeffs_d,
@@ -165,12 +151,12 @@ extern "C" int b200ldu_fvm_H(b200ldu_matrix *m, int nComp, const double *psi_d, 
     }
     if (nComp == 1)
         H_kernel<1><<<grid(a->nCells, 128), 128, 0, a->ctx->stream>>>(
-            a->nCells, a->d_ownerStart, a->d_u, a->d_losortStart, a->d_losort, a->d_l, m->upper_ext, m->lower_ext, L,
-            boundaryCoeffs_d, m->bou_ext, pnf_d, psi_d, source_d, V_d, H_d);
+            a->nCells, a->d_ownerStart.get(), a->d_u.get(), a->d_losortStart.get(), a->d_losort.get(), a->d_l.get(),
+            m->upper_ext, m->lower_ext, L, boundaryCoeffs_d, m->bou_ext, pnf_d, psi_d, source_d, V_d, H_d);
     else
         H_kernel<3><<<grid(a->nCells, 128), 128, 0, a->ctx->stream>>>(
-            a->nCells, a->d_ownerStart, a->d_u, a->d_losortStart, a->d_losort, a->d_l, m->upper_ext, m->lower_ext, L,
-            boundaryCoeffs_d, m->bou_ext, pnf_d, psi_d, source_d, V_d, H_d);
+            a->nCells, a->d_ownerStart.get(), a->d_u.get(), a->d_losortStart.get(), a->d_losort.get(), a->d_l.get(),
+            m->upper_ext, m->lower_ext, L, boundaryCoeffs_d, m->bou_ext, pnf_d, psi_d, source_d, V_d, H_d);
     a->ctx->launches++;
     KERNEL_CHECK();
     return B200LDU_OK;
@@ -194,30 +180,30 @@ extern "C" int b200ldu_fvm_flux(b200ldu_matrix *m, int nComp, const double *psi_
     cudaStream_t st = a->ctx->stream;
     if (a->nFaces) {
         if (nComp == 1)
-            flux_internal_kernel<1><<<grid(a->nFaces, 256), 256, 0, st>>>(a->nFaces, a->d_l, a->d_u, m->upper_ext,
+            flux_internal_kernel<1><<<grid(a->nFaces, 256), 256, 0, st>>>(a->nFaces, a->d_l.get(), a->d_u.get(), m->upper_ext,
                                                                           m->lower_ext, psi_d, flux_d);
         else
-            flux_internal_kernel<3><<<grid(a->nFaces, 256), 256, 0, st>>>(a->nFaces, a->d_l, a->d_u, m->upper_ext,
+            flux_internal_kernel<3><<<grid(a->nFaces, 256), 256, 0, st>>>(a->nFaces, a->d_l.get(), a->d_u.get(), m->upper_ext,
                                                                           m->lower_ext, psi_d, flux_d);
         a->ctx->launches++;
     }
     if (a->nBFaces) {
         if (nComp == 1)
-            flux_boundary_kernel<1><<<grid(a->nBFaces, 256), 256, 0, st>>>(a->nBFaces, a->d_bFaceCells, internalCoeffs_d,
+            flux_boundary_kernel<1><<<grid(a->nBFaces, 256), 256, 0, st>>>(a->nBFaces, a->d_bFaceCells.get(), internalCoeffs_d,
                                                                            1, boundaryCoeffs_d, 1, nullptr, psi_d,
                                                                            boundaryFlux_d);
         else
-            flux_boundary_kernel<3><<<grid(a->nBFaces, 256), 256, 0, st>>>(a->nBFaces, a->d_bFaceCells, internalCoeffs_d,
+            flux_boundary_kernel<3><<<grid(a->nBFaces, 256), 256, 0, st>>>(a->nBFaces, a->d_bFaceCells.get(), internalCoeffs_d,
                                                                            3, boundaryCoeffs_d, 3, nullptr, psi_d,
                                                                            boundaryFlux_d);
         a->ctx->launches++;
     }
     if (a->nCFaces) {
         if (nComp == 1)
-            flux_boundary_kernel<1><<<grid(a->nCFaces, 256), 256, 0, st>>>(a->nCFaces, a->d_cFaceCells, m->int_ext, 1,
+            flux_boundary_kernel<1><<<grid(a->nCFaces, 256), 256, 0, st>>>(a->nCFaces, a->d_cFaceCells.get(), m->int_ext, 1,
                                                                            m->bou_ext, 1, pnf_d, psi_d, coupledFlux_d);
         else
-            flux_boundary_kernel<3><<<grid(a->nCFaces, 256), 256, 0, st>>>(a->nCFaces, a->d_cFaceCells, m->int_ext, 1,
+            flux_boundary_kernel<3><<<grid(a->nCFaces, 256), 256, 0, st>>>(a->nCFaces, a->d_cFaceCells.get(), m->int_ext, 1,
                                                                            m->bou_ext, 1, pnf_d, psi_d, coupledFlux_d);
         a->ctx->launches++;
     }
@@ -240,13 +226,13 @@ extern "C" int b200ldu_fvm_residual(b200ldu_matrix *m, const double *psi_d, cons
         b200_set_error("fvm_residual: the coupled patches need their patchNeighbourField (addBoundarySource)");
         return B200LDU_EINVAL;
     }
-    double *tmp = nullptr;
-    TRY(scratch(a, 0, (size_t)a->nCells, &tmp));
+    DevBuf<double> &tmp = a->fvmScratch[FVM_DIAG];
+    TRY(tmp.grow((size_t)a->nCells));
     residual_source_kernel<<<grid(a->nCells, 256), 256, 0, a->ctx->stream>>>(a->nCells, L, internalCoeffs_d, m->int_ext,
-                                                                             psi_d, source_d, tmp);
+                                                                             psi_d, source_d, tmp.get());
     a->ctx->launches++;
     KERNEL_CHECK();
-    TRY(b200ldu_residual(m, psi_d, tmp, residual_d)); // lduMatrix::residual incl. the interface update
+    TRY(b200ldu_residual(m, psi_d, tmp.get(), residual_d)); // lduMatrix::residual incl. the interface update
     return b200ldu_fvm_add_boundary_source(m, 1, boundaryCoeffs_d, pnf_d, residual_d, residual_d);
 }
 
@@ -262,12 +248,12 @@ extern "C" int b200ldu_fvm_relax(b200ldu_matrix *m, int nComp, double alpha, con
     TRY(lists(a, &L));
     if (nComp == 1)
         relax_kernel<1><<<grid(a->nCells, 128), 128, 0, a->ctx->stream>>>(
-            a->nCells, a->d_ownerStart, a->d_losortStart, a->d_losort, m->upper_ext, m->lower_ext, L, internalCoeffs_d,
-            m->int_ext, m->bou_ext, alpha, psi_d, diag_d, source_d);
+            a->nCells, a->d_ownerStart.get(), a->d_losortStart.get(), a->d_losort.get(), m->upper_ext, m->lower_ext, L,
+            internalCoeffs_d, m->int_ext, m->bou_ext, alpha, psi_d, diag_d, source_d);
     else
         relax_kernel<3><<<grid(a->nCells, 128), 128, 0, a->ctx->stream>>>(
-            a->nCells, a->d_ownerStart, a->d_losortStart, a->d_losort, m->upper_ext, m->lower_ext, L, internalCoeffs_d,
-            m->int_ext, m->bou_ext, alpha, psi_d, diag_d, source_d);
+            a->nCells, a->d_ownerStart.get(), a->d_losortStart.get(), a->d_losort.get(), m->upper_ext, m->lower_ext, L,
+            internalCoeffs_d, m->int_ext, m->bou_ext, alpha, psi_d, diag_d, source_d);
     a->ctx->launches++;
     KERNEL_CHECK();
     return B200LDU_OK;
@@ -311,9 +297,10 @@ extern "C" int b200ldu_fvm_solve(b200ldu_matrix *m, int nComp, const char *solve
     // the caller's coefficient arrays: the matrix is re-pointed at the folded diagonal for the solve
     const double *diag0 = m->diag_ext;
     const double *bou = m->bou_ext, *intc = m->int_ext;
-    double *dK = nullptr, *total = nullptr, *sK = nullptr, *pK = nullptr;
-    TRY(scratch(a, 0, (size_t)n, &dK));
-    TRY(scratch(a, 1, (size_t)n * nComp, &total));
+    DevBuf<double> *scr = a->fvmScratch;
+    TRY(scr[FVM_DIAG].grow((size_t)n));
+    TRY(scr[FVM_SOURCE].grow((size_t)n * nComp));
+    double *dK = scr[FVM_DIAG].get(), *total = scr[FVM_SOURCE].get();
     int rc = B200LDU_OK;
     if (nComp == 1) {
         boundary_diag_kernel<<<grid(n, 256), 256, 0, st>>>(n, L, internalCoeffs_d, 1, 0, intc, diag0, dK);
@@ -323,8 +310,9 @@ extern "C" int b200ldu_fvm_solve(b200ldu_matrix *m, int nComp, const char *solve
         rc = matrix_set_diag(m, dK); // the off-diagonal streams are unchanged
         if (rc == B200LDU_OK) rc = b200ldu_solve(m, solver, precondOrSmoother, controls, gamg, psi_d, total, &perf[0], nullptr, 0);
     } else {
-        TRY(scratch(a, 2, (size_t)n, &sK));
-        TRY(scratch(a, 3, (size_t)n, &pK));
+        TRY(scr[FVM_CMPT_SOURCE].grow((size_t)n));
+        TRY(scr[FVM_CMPT_PSI].grow((size_t)n));
+        double *sK = scr[FVM_CMPT_SOURCE].get(), *pK = scr[FVM_CMPT_PSI].get();
         boundary_source_kernel<3><<<grid(n, 256), 256, 0, st>>>(n, L, boundaryCoeffs_d, bou, pnf_d, source_d, total);
         a->ctx->launches++;
         KERNEL_CHECK();

@@ -38,35 +38,37 @@ struct GamgLevel {
     std::vector<int> restrictAddr;      // fine cell -> coarse cell (caller orders)
     std::vector<int> faceRestrict;      // fine face -> coarse face | -(cell+1)
     std::vector<unsigned char> faceFlip;
-    b200ldu_addr *addr = nullptr;       // coarse level addressing (banded layout built)
-    b200ldu_matrix *mat = nullptr;      // coarse level matrix (values refreshed every solve)
+    // coarse level addressing (banded layout built) and matrix (values refreshed every solve): the matrix is
+    // declared after the addressing so that it is destroyed first
+    AbiHandle<b200ldu_addr, b200ldu_addr_destroy> addr;
+    AbiHandle<b200ldu_matrix, b200ldu_matrix_destroy> mat;
     // device maps, banded vector space
-    int *d_childStart = nullptr, *d_child = nullptr; // coarse banded row -> fine banded rows (asc. fine cell)
-    int *d_pmap = nullptr;                           // fine banded row -> coarse banded row (-1 padding)
+    DevBuf<int> d_childStart, d_child; // coarse banded row -> fine banded rows (asc. fine cell)
+    DevBuf<int> d_pmap;                // fine banded row -> coarse banded row (-1 padding)
     // device maps, caller order (coefficients)
-    int *d_cellChildStart = nullptr, *d_cellChild = nullptr; // coarse cell -> fine cells ascending
-    int *d_faceChildStart = nullptr, *d_faceChild = nullptr; // coarse face -> (fine face << 1 | flip) ascending
-    int *d_diagFaceStart = nullptr, *d_diagFace = nullptr;   // coarse cell -> collapsed fine faces ascending
-    double *d_diag = nullptr, *d_upper = nullptr, *d_lower = nullptr; // caller-order coarse coefficients
+    DevBuf<int> d_cellChildStart, d_cellChild; // coarse cell -> fine cells ascending
+    DevBuf<int> d_faceChildStart, d_faceChild; // coarse face -> (fine face << 1 | flip) ascending
+    DevBuf<int> d_diagFaceStart, d_diagFace;   // coarse cell -> collapsed fine faces ascending
+    DevBuf<double> d_diag, d_upper, d_lower;   // caller-order coarse coefficients
     // coupled patches of the coarse level
     int nFinePF = 0, nCoarsePF = 0;
     std::vector<int> cPatchStart, cFaceCells;
-    int *d_pfChildStart = nullptr, *d_pfChild = nullptr; // coarse patch face -> fine patch faces ascending
-    double *d_bou = nullptr, *d_int = nullptr;
+    DevBuf<int> d_pfChildStart, d_pfChild; // coarse patch face -> fine patch faces ascending
+    DevBuf<double> d_bou, d_int;
     // level vectors (banded, vecLen of the coarse level)
-    double *corr = nullptr, *src = nullptr, *tmp = nullptr, *acf = nullptr, *pre = nullptr;
+    DevBuf<double> corr, src, tmp, acf, pre;
 };
 
 struct b200ldu_gamg {
     b200ldu_addr *finest = nullptr;
     int nLevels = 0;
     std::vector<GamgLevel> lev;
-    double *d_inv = nullptr; // this rank's rows of the inverse of the (global) coarsest matrix
-    int invN = 0;            // global size of the coarsest system
+    DevBuf<double> d_inv; // this rank's rows of the inverse of the (global) coarsest matrix
+    int invN = 0;         // global size of the coarsest system
     // multi-rank coarsest solve
     std::vector<int> coarsestCounts, coarsestOffs, coarsestNbrCell;
     int nMaxCoarsest = 0;
-    double *d_gatherAll = nullptr; // NCCL fallback of the peer-memory gather
+    DevBuf<double> d_gatherAll; // NCCL fallback of the peer-memory gather
     bool metaUploaded = false;
 };
 
@@ -198,25 +200,11 @@ static void csr_from_map(const std::vector<int> &map, int nTargets, std::vector<
         if (map[i] >= 0) items[cur[map[i]]++] = i;
 }
 
-static void level_free(GamgLevel &L)
-{
-    void *ptrs[] = {L.d_childStart, L.d_child, L.d_pmap, L.d_cellChildStart, L.d_cellChild, L.d_faceChildStart,
-                    L.d_faceChild, L.d_diagFaceStart, L.d_diagFace, L.d_diag, L.d_upper, L.d_lower,
-                    L.corr, L.src, L.tmp, L.acf, L.pre, L.d_pfChildStart, L.d_pfChild, L.d_bou, L.d_int};
-    for (void *p : ptrs)
-        if (p) cudaFree(p);
-    if (L.mat) b200ldu_matrix_destroy(L.mat);
-    if (L.addr) b200ldu_addr_destroy(L.addr);
-}
-
 extern "C" int b200ldu_gamg_destroy(b200ldu_gamg *g)
 {
     if (!g) return B200LDU_OK;
     cudaSetDevice(g->finest->ctx->device);
     cudaStreamSynchronize(g->finest->ctx->stream);
-    for (auto &L : g->lev) level_free(L);
-    if (g->d_inv) cudaFree(g->d_inv);
-    if (g->d_gatherAll) cudaFree(g->d_gatherAll);
     delete g;
     return B200LDU_OK;
 }
@@ -235,7 +223,7 @@ extern "C" int b200ldu_gamg_create(b200ldu_addr *a, const double *faceWeights_h,
             return B200LDU_EINVAL;
         }
     CUDA_TRY(cudaSetDevice(a->ctx->device));
-    b200ldu_gamg *g = new b200ldu_gamg();
+    AbiHandle<b200ldu_gamg, b200ldu_gamg_destroy> g(new b200ldu_gamg());
     g->finest = a;
     bool forward = forwardInOut ? (*forwardInOut != 0) : true; // pairGAMGAgglomeration.C:33
     std::vector<int> lo = a->l, up = a->u;
@@ -260,7 +248,7 @@ extern "C" int b200ldu_gamg_create(b200ldu_addr *a, const double *faceWeights_h,
     auto finalize = [&](HostStep &H) -> int {
         g->lev.emplace_back();
         GamgLevel &L = g->lev.back();
-        b200ldu_addr *fineAddr = g->lev.size() >= 2 ? g->lev[g->lev.size() - 2].addr : a;
+        b200ldu_addr *fineAddr = g->lev.size() >= 2 ? g->lev[g->lev.size() - 2].addr.get() : a;
         const std::vector<int> &finePerm = fineAddr->perm_h, &fiperm = fineAddr->iperm_h;
         L.nFine = H.nFine;
         L.nFineFaces = H.nFineFaces;
@@ -275,29 +263,28 @@ extern "C" int b200ldu_gamg_create(b200ldu_addr *a, const double *faceWeights_h,
         L.cFaceCells.swap(H.cFaceCells);
         const std::vector<int> &map = L.restrictAddr;
         const int nCoarse = L.nCoarse, nFineL = L.nFine;
-        int r = b200ldu_addr_create(a->ctx, nCoarse, L.nCoarseFaces, H.cOwner.data(), H.cNeigh.data(), nPatches,
-                                    nPatches ? L.cPatchStart.data() : nullptr, nPatches ? L.cFaceCells.data() : nullptr,
-                                    nPatches ? a->neighbRank.data() : nullptr, H.cc.empty() ? nullptr : H.cc.data(),
-                                    &L.addr);
-        if (r != B200LDU_OK) return r;
+        b200ldu_addr *ca = nullptr;
+        TRY(b200ldu_addr_create(a->ctx, nCoarse, L.nCoarseFaces, H.cOwner.data(), H.cNeigh.data(), nPatches,
+                                nPatches ? L.cPatchStart.data() : nullptr, nPatches ? L.cFaceCells.data() : nullptr,
+                                nPatches ? a->neighbRank.data() : nullptr, H.cc.empty() ? nullptr : H.cc.data(), &ca));
+        L.addr.reset(ca);
         if (nPatches) {
             std::vector<int> ps, pi;
             csr_from_map(H.pfRestrict, L.nCoarsePF, ps, pi);
-            TRY(dev_upload(&L.d_pfChildStart, ps));
-            TRY(dev_upload(&L.d_pfChild, pi));
-            if (cudaMalloc((void **)&L.d_bou, sizeof(double) * (size_t)std::max(L.nCoarsePF, 1)) != cudaSuccess ||
-                cudaMalloc((void **)&L.d_int, sizeof(double) * (size_t)std::max(L.nCoarsePF, 1)) != cudaSuccess) {
-                b200_set_error("GAMG: out of device memory");
-                return B200LDU_ECUDA;
-            }
+            TRY(L.d_pfChildStart.upload(ps));
+            TRY(L.d_pfChild.upload(pi));
+            TRY(L.d_bou.alloc((size_t)std::max(L.nCoarsePF, 1)));
+            TRY(L.d_int.alloc((size_t)std::max(L.nCoarsePF, 1)));
         }
-        TRY(b200ldu_matrix_create(L.addr, &L.mat));
+        b200ldu_matrix *cm = nullptr;
+        TRY(b200ldu_matrix_create(L.addr.get(), &cm));
+        L.mat.reset(cm);
         // ---- device maps ----
         {
             std::vector<int> cs, ci;
             csr_from_map(map, nCoarse, cs, ci); // coarse cell -> fine cells ascending
-            TRY(dev_upload(&L.d_cellChildStart, cs));
-            TRY(dev_upload(&L.d_cellChild, ci));
+            TRY(L.d_cellChildStart.upload(cs));
+            TRY(L.d_cellChild.upload(ci));
             // banded versions
             const std::vector<int> &cperm = L.addr->perm_h, &ciperm = L.addr->iperm_h;
             const int nPadC = L.addr->L.nPad, nPadF = fineAddr->L.nPad;
@@ -311,9 +298,9 @@ extern "C" int b200ldu_gamg_create(b200ldu_addr *a, const double *faceWeights_h,
             std::vector<int> pm(nPadF, -1);
             for (int q = 0; q < nPadF; q++)
                 if (fiperm[q] >= 0) pm[q] = cperm[map[fiperm[q]]];
-            TRY(dev_upload(&L.d_childStart, bs));
-            TRY(dev_upload(&L.d_child, bi));
-            TRY(dev_upload(&L.d_pmap, pm));
+            TRY(L.d_childStart.upload(bs));
+            TRY(L.d_child.upload(bi));
+            TRY(L.d_pmap.upload(pm));
             // face maps (caller order)
             std::vector<int> fmap(L.nFineFaces), dmap(L.nFineFaces);
             for (int f = 0; f < L.nFineFaces; f++) {
@@ -324,19 +311,16 @@ extern "C" int b200ldu_gamg_create(b200ldu_addr *a, const double *faceWeights_h,
             csr_from_map(fmap, L.nCoarseFaces, fs, fi);
             csr_from_map(dmap, nCoarse, ds, di);
             for (int k = 0; k < fs[L.nCoarseFaces]; k++) fi[k] = (fi[k] << 1) | (L.faceFlip[fi[k]] ? 1 : 0);
-            TRY(dev_upload(&L.d_faceChildStart, fs));
-            TRY(dev_upload(&L.d_faceChild, fi));
-            TRY(dev_upload(&L.d_diagFaceStart, ds));
-            TRY(dev_upload(&L.d_diagFace, di));
+            TRY(L.d_faceChildStart.upload(fs));
+            TRY(L.d_faceChild.upload(fi));
+            TRY(L.d_diagFaceStart.upload(ds));
+            TRY(L.d_diagFace.upload(di));
         }
         size_t nf = (size_t)std::max(L.nCoarseFaces, 1);
-        if (cudaMalloc((void **)&L.d_diag, sizeof(double) * (size_t)nCoarse) != cudaSuccess ||
-            cudaMalloc((void **)&L.d_upper, sizeof(double) * nf) != cudaSuccess ||
-            cudaMalloc((void **)&L.d_lower, sizeof(double) * nf) != cudaSuccess) {
-            b200_set_error("GAMG: out of device memory");
-            return B200LDU_ECUDA;
-        }
-        for (double **v : {&L.corr, &L.src, &L.tmp, &L.acf, &L.pre}) TRY(addr_alloc_vec(L.addr, v));
+        TRY(L.d_diag.alloc((size_t)nCoarse));
+        TRY(L.d_upper.alloc(nf));
+        TRY(L.d_lower.alloc(nf));
+        for (DevBuf<double> *v : {&L.corr, &L.src, &L.tmp, &L.acf, &L.pre}) TRY(addr_alloc_vec(L.addr.get(), *v));
         return B200LDU_OK;
     };
 
@@ -465,10 +449,7 @@ extern "C" int b200ldu_gamg_create(b200ldu_addr *a, const double *faceWeights_h,
     }
     if (rc == B200LDU_OK && havePend) rc = finalize(pend);
     if (forwardInOut) *forwardInOut = forward ? 1 : 0;
-    if (rc != B200LDU_OK) {
-        b200ldu_gamg_destroy(g);
-        return rc;
-    }
+    if (rc != B200LDU_OK) return rc;
     g->nLevels = (int)g->lev.size();
     // coarsest level across the ranks: sizes, offsets and the neighbour-side cell of every
     // coarsest processor-patch face (columns of the global matrix, LUscalarMatrix.C:201-270)
@@ -498,12 +479,9 @@ extern "C" int b200ldu_gamg_create(b200ldu_addr *a, const double *faceWeights_h,
             rc = comm_exchange_patch_ints(a->ctx, nPatches, LC.cPatchStart.data(), a->neighbRank.data(),
                                           LC.cFaceCells.data(), g->coarsestNbrCell.data());
         }
-        if (rc != B200LDU_OK) {
-            b200ldu_gamg_destroy(g);
-            return rc;
-        }
+        if (rc != B200LDU_OK) return rc;
     }
-    *out = g;
+    *out = g.release();
     return B200LDU_OK;
 }
 
@@ -701,11 +679,11 @@ struct LevelView { // uniform access to the finest matrix (-1) and coarse level 
     b200ldu_matrix *m;
 };
 
-int smooth_in_place(Solve &S, b200ldu_matrix *m, double omega, double *&x, double *&spare, const double *b,
-                    int nSweeps, const int *stop)
+int smooth_in_place(Solve &S, b200ldu_matrix *m, double omega, DevBuf<double> &x, DevBuf<double> &spare,
+                    const double *b, int nSweeps, const int *stop)
 {
     for (int s = 0; s < nSweeps; s++) {
-        TRY(mat_jacobi(m, omega, x, b, spare, stop));
+        TRY(mat_jacobi(m, omega, x.get(), b, spare.get(), stop));
         std::swap(x, spare);
     }
     return B200LDU_OK;
@@ -715,13 +693,13 @@ int smooth_in_place(Solve &S, b200ldu_matrix *m, double omega, double *&x, doubl
 int gamg_scale(Solve &S, b200ldu_matrix *m, double *field, double *Acf, const double *source, const int *stop)
 {
     SolverScalars *sc = S.sc;
-    TRY(mat_amul(m, false, field, Acf, 2, source, m->d_partials, stop));
-    TRY(scalar_step_on<2>(S, m->d_partials, m->a->L.nBands, [=] __device__(SolverScalars *s) {
+    TRY(mat_amul(m, false, field, Acf, 2, source, m->d_partials.get(), stop));
+    TRY(scalar_step_on<2>(S, m->d_partials.get(), m->a->L.nBands, [=] __device__(SolverScalars *s) {
         double den = s->sum[1];
         double sden = den >= 0 ? den + VSMALL_ : den - VSMALL_; // stabilise(y, VSMALL)
         s->alpha = s->sum[0] / sden;
     }));
-    const double *D = m->d_diag;
+    const double *D = m->d_diag.get();
     return ew_launch<0>(S.ctx, m->a->L.nPad / 2, stop, nullptr, nullptr, [=] __device__(int i, double *) {
         double sf = sc->alpha;
         double2 f = CV2(field)[i], a = CV2(Acf)[i], b = CV2(source)[i], d = CV2(D)[i];
@@ -747,24 +725,24 @@ static int gamg_build_matrices(Solve &S, b200ldu_gamg *g)
     }
     for (int k = 0; k < g->nLevels; k++) {
         GamgLevel &L = g->lev[k];
-        LAUNCH1D(agg_diag_kernel, L.nCoarse, st, L.nCoarse, L.d_cellChildStart, L.d_cellChild, L.d_diagFaceStart,
-                 L.d_diagFace, fd, fu, fl, L.d_diag);
-        LAUNCH1D(agg_faces_kernel, L.nCoarseFaces, st, L.nCoarseFaces, L.d_faceChildStart, L.d_faceChild, fu, fl,
-                 L.d_upper, L.d_lower);
+        LAUNCH1D(agg_diag_kernel, L.nCoarse, st, L.nCoarse, L.d_cellChildStart.get(), L.d_cellChild.get(),
+                 L.d_diagFaceStart.get(), L.d_diagFace.get(), fd, fu, fl, L.d_diag.get());
+        LAUNCH1D(agg_faces_kernel, L.nCoarseFaces, st, L.nCoarseFaces, L.d_faceChildStart.get(), L.d_faceChild.get(),
+                 fu, fl, L.d_upper.get(), L.d_lower.get());
         if (L.nCoarsePF > 0) {
-            LAUNCH1D(agg_patch_kernel, L.nCoarsePF, st, L.nCoarsePF, L.d_pfChildStart, L.d_pfChild, fb, fi, L.d_bou,
-                     L.d_int);
+            LAUNCH1D(agg_patch_kernel, L.nCoarsePF, st, L.nCoarsePF, L.d_pfChildStart.get(), L.d_pfChild.get(), fb, fi,
+                     L.d_bou.get(), L.d_int.get());
         }
         KERNEL_CHECK();
         // identical boundary/internal interface coefficients on the finest level stay identical
-        const double *cInt = (fm->bou_ext == fm->int_ext) ? L.d_bou : L.d_int;
-        TRY(b200ldu_matrix_set(L.mat, L.d_diag, L.d_upper, fl ? L.d_lower : nullptr, L.nCoarsePF > 0 ? L.d_bou : nullptr,
-                               L.nCoarsePF > 0 ? cInt : nullptr));
-        fb = L.d_bou;
-        fi = L.d_int;
-        fd = L.d_diag;
-        fu = L.d_upper;
-        fl = fl ? L.d_lower : nullptr;
+        const double *cInt = (fm->bou_ext == fm->int_ext) ? L.d_bou.get() : L.d_int.get();
+        TRY(b200ldu_matrix_set(L.mat.get(), L.d_diag.get(), L.d_upper.get(), fl ? L.d_lower.get() : nullptr,
+                               L.nCoarsePF > 0 ? L.d_bou.get() : nullptr, L.nCoarsePF > 0 ? cInt : nullptr));
+        fb = L.d_bou.get();
+        fi = L.d_int.get();
+        fd = L.d_diag.get();
+        fu = L.d_upper.get();
+        fl = fl ? L.d_lower.get() : nullptr;
     }
     return B200LDU_OK;
 }
@@ -783,10 +761,10 @@ static int gamg_coarsest_inverse(Solve &S, b200ldu_gamg *g)
     bool asym = !S.m->symmetric;
     std::vector<double> d(std::max(n, 1)), u(std::max(nf, 1)), l(std::max(nf, 1)), bou(std::max(npf, 1));
     cudaStream_t st = ctx->stream;
-    CUDA_TRY(cudaMemcpyAsync(d.data(), L.d_diag, sizeof(double) * n, cudaMemcpyDeviceToHost, st));
-    if (nf) CUDA_TRY(cudaMemcpyAsync(u.data(), L.d_upper, sizeof(double) * nf, cudaMemcpyDeviceToHost, st));
-    if (nf && asym) CUDA_TRY(cudaMemcpyAsync(l.data(), L.d_lower, sizeof(double) * nf, cudaMemcpyDeviceToHost, st));
-    if (npf) CUDA_TRY(cudaMemcpyAsync(bou.data(), L.d_bou, sizeof(double) * npf, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(d.data(), L.d_diag.get(), sizeof(double) * n, cudaMemcpyDeviceToHost, st));
+    if (nf) CUDA_TRY(cudaMemcpyAsync(u.data(), L.d_upper.get(), sizeof(double) * nf, cudaMemcpyDeviceToHost, st));
+    if (nf && asym) CUDA_TRY(cudaMemcpyAsync(l.data(), L.d_lower.get(), sizeof(double) * nf, cudaMemcpyDeviceToHost, st));
+    if (npf) CUDA_TRY(cudaMemcpyAsync(bou.data(), L.d_bou.get(), sizeof(double) * npf, cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     if (!asym) l = u;
     const std::vector<int> &perm = L.addr->perm_h;
@@ -864,16 +842,11 @@ static int gamg_coarsest_inverse(Solve &S, b200ldu_gamg *g)
             }
         }
     }
-    size_t need = (size_t)std::max(n, 1) * N;
-    if ((size_t)g->invN * g->invN < need || !g->d_inv) {
-        if (g->d_inv) cudaFree(g->d_inv);
-        g->d_inv = nullptr;
-        CUDA_TRY(cudaMalloc((void **)&g->d_inv, sizeof(double) * need));
-    }
+    TRY(g->d_inv.grow((size_t)std::max(n, 1) * N));
     g->invN = N;
-    CUDA_TRY(cudaMemcpyAsync(g->d_inv, &I[(size_t)off * N], sizeof(double) * (size_t)n * N, cudaMemcpyHostToDevice, st));
-    if (R > 1 && !ctx->p2p && !g->d_gatherAll)
-        CUDA_TRY(cudaMalloc((void **)&g->d_gatherAll, sizeof(double) * (size_t)(R + 1) * P2P_GMAX + sizeof(int) * 64));
+    CUDA_TRY(cudaMemcpyAsync(g->d_inv.get(), &I[(size_t)off * N], sizeof(double) * (size_t)n * N, cudaMemcpyHostToDevice, st));
+    if (R > 1 && !ctx->p2p) // R + 1 gather rows, then 64 ints of offsets and counts
+        TRY(g->d_gatherAll.grow((size_t)(R + 1) * P2P_GMAX + sizeof(int) * 64 / sizeof(double)));
     CUDA_TRY(cudaStreamSynchronize(st)); // I goes out of scope
     return B200LDU_OK;
 }
@@ -911,29 +884,29 @@ static int gamg_cycle(void *vp)
     // ---- Vcycle (GAMGSolverSolve.C:181-474) ----
     {
         GamgLevel &L0 = g->lev[0];
-        LAUNCH1D(restrict_kernel, L0.nCoarse, st, L0.nCoarse, L0.d_childStart, L0.d_child, A.finestRes, L0.src, stop);
+        LAUNCH1D(restrict_kernel, L0.nCoarse, st, L0.nCoarse, L0.d_childStart.get(), L0.d_child.get(), A.finestRes, L0.src.get(), stop);
     }
     for (int k = 0; k < coarsest; k++) {
         GamgLevel &L = g->lev[k], &Ln = g->lev[k + 1];
         if (c.nPreSweeps) {
-            CUDA_TRY(cudaMemsetAsync(L.corr, 0, sizeof(double) * (size_t)L.addr->vecLen, st));
-            TRY(smooth_in_place(S, L.mat, omega, L.corr, L.tmp, L.src,
+            CUDA_TRY(cudaMemsetAsync(L.corr.get(), 0, sizeof(double) * (size_t)L.addr->vecLen, st));
+            TRY(smooth_in_place(S, L.mat.get(), omega, L.corr, L.tmp, L.src.get(),
                                 imin(c.nPreSweeps + c.preSweepsLevelMultiplier * k, c.maxPreSweeps), stop));
-            if (A.scaleCorrection && k < coarsest - 1) TRY(gamg_scale(S, L.mat, L.corr, L.acf, L.src, stop));
-            TRY(mat_amul(L.mat, false, L.corr, L.acf, 0, nullptr, nullptr, stop));
-            double *src = L.src, *acf = L.acf;
+            if (A.scaleCorrection && k < coarsest - 1) TRY(gamg_scale(S, L.mat.get(), L.corr.get(), L.acf.get(), L.src.get(), stop));
+            TRY(mat_amul(L.mat.get(), false, L.corr.get(), L.acf.get(), 0, nullptr, nullptr, stop));
+            double *src = L.src.get(), *acf = L.acf.get();
             TRY(ew_launch<0>(S.ctx, L.addr->L.nPad / 2, stop, nullptr, nullptr, [=] __device__(int i, double *) {
                 double2 s2 = CV2(src)[i], a2 = CV2(acf)[i];
                 V2(src)[i] = make_double2(__dsub_rn(s2.x, a2.x), __dsub_rn(s2.y, a2.y));
             }));
         }
-        LAUNCH1D(restrict_kernel, Ln.nCoarse, st, Ln.nCoarse, Ln.d_childStart, Ln.d_child, L.src, Ln.src, stop);
+        LAUNCH1D(restrict_kernel, Ln.nCoarse, st, Ln.nCoarse, Ln.d_childStart.get(), Ln.d_child.get(), L.src.get(), Ln.src.get(), stop);
     }
     { // solveCoarsestLevel :552-619
         GamgLevel &L = g->lev[coarsest];
         if (c.directSolveCoarsest) {
             if (S.ctx->nRanks == 1) {
-                dense_apply_kernel<<<1, 256, 0, st>>>(L.nCoarse, g->d_inv, L.src, L.corr, stop);
+                dense_apply_kernel<<<1, 256, 0, st>>>(L.nCoarse, g->d_inv.get(), L.src.get(), L.corr.get(), stop);
             } else if (S.ctx->p2p) {
                 P2PGather G;
                 G.rank = S.ctx->rank;
@@ -945,15 +918,15 @@ static int gamg_cycle(void *vp)
                     G.offs[r] = g->coarsestOffs[r];
                 }
                 G.offs[G.nRanks] = g->coarsestOffs[G.nRanks];
-                G.seq = S.ctx->d_seq + 2;
-                dense_apply_p2p_kernel<<<1, 256, 0, st>>>(L.nCoarse, g->invN, g->d_inv, L.src, L.corr, G, stop);
+                G.seq = S.ctx->d_seq.get() + 2;
+                dense_apply_p2p_kernel<<<1, 256, 0, st>>>(L.nCoarse, g->invN, g->d_inv.get(), L.src.get(), L.corr.get(), G, stop);
             } else {
                 // NCCL fallback: pad to P2P_GMAX per rank, all-gather, apply
-                double *mine = g->d_gatherAll + (size_t)S.ctx->nRanks * P2P_GMAX;
+                double *mine = g->d_gatherAll.get() + (size_t)S.ctx->nRanks * P2P_GMAX;
                 CUDA_TRY(cudaMemsetAsync(mine, 0, sizeof(double) * P2P_GMAX, st));
-                CUDA_TRY(cudaMemcpyAsync(mine, L.src, sizeof(double) * L.nCoarse, cudaMemcpyDeviceToDevice, st));
-                TRY(comm_allgather_dev(S.ctx, mine, P2P_GMAX, g->d_gatherAll));
-                int *meta = (int *)(g->d_gatherAll + (size_t)(S.ctx->nRanks + 1) * P2P_GMAX);
+                CUDA_TRY(cudaMemcpyAsync(mine, L.src.get(), sizeof(double) * L.nCoarse, cudaMemcpyDeviceToDevice, st));
+                TRY(comm_allgather_dev(S.ctx, mine, P2P_GMAX, g->d_gatherAll.get()));
+                int *meta = (int *)(g->d_gatherAll.get() + (size_t)(S.ctx->nRanks + 1) * P2P_GMAX);
                 if (!g->metaUploaded) {
                     std::vector<int> h(64, 0);
                     for (int r = 0; r <= S.ctx->nRanks; r++) h[r] = g->coarsestOffs[r];
@@ -962,8 +935,8 @@ static int gamg_cycle(void *vp)
                     CUDA_TRY(cudaStreamSynchronize(st));
                     g->metaUploaded = true;
                 }
-                dense_apply_gathered_kernel<<<1, 256, 0, st>>>(L.nCoarse, g->invN, S.ctx->nRanks, g->d_inv, g->d_gatherAll,
-                                                                meta, meta + 32, L.corr, stop);
+                dense_apply_gathered_kernel<<<1, 256, 0, st>>>(L.nCoarse, g->invN, S.ctx->nRanks, g->d_inv.get(),
+                                                                g->d_gatherAll.get(), meta, meta + 32, L.corr.get(), stop);
             }
             S.ctx->launches++;
         } else {
@@ -974,17 +947,17 @@ static int gamg_cycle(void *vp)
             CUDA_TRY(cudaMemcpyAsync(&stopped, stop, sizeof(int), cudaMemcpyDeviceToHost, st));
             CUDA_TRY(cudaStreamSynchronize(st));
             if (!stopped) {
-                CUDA_TRY(cudaMemsetAsync(L.corr, 0, sizeof(double) * (size_t)L.addr->vecLen, st));
+                CUDA_TRY(cudaMemsetAsync(L.corr.get(), 0, sizeof(double) * (size_t)L.addr->vecLen, st));
                 b200ldu_controls cc;
                 b200ldu_controls_default(&cc);
                 cc.tolerance = c.tolerance;
                 cc.relTol = c.relTol;
                 b200ldu_perf cp;
                 double *res = nullptr;
-                TRY(solve_banded(L.mat, L.mat->symmetric ? "ICCG" : "BICCG", nullptr, &cc, nullptr, L.corr, L.src, &cp,
-                                 nullptr, 0, &res));
-                if (res != L.corr)
-                    CUDA_TRY(cudaMemcpyAsync(L.corr, res, sizeof(double) * (size_t)L.addr->vecLen,
+                TRY(solve_banded(L.mat.get(), L.mat->symmetric ? "ICCG" : "BICCG", nullptr, &cc, nullptr, L.corr.get(),
+                                 L.src.get(), &cp, nullptr, 0, &res));
+                if (res != L.corr.get())
+                    CUDA_TRY(cudaMemcpyAsync(L.corr.get(), res, sizeof(double) * (size_t)L.addr->vecLen,
                                              cudaMemcpyDeviceToDevice, st));
             }
         }
@@ -993,28 +966,28 @@ static int gamg_cycle(void *vp)
         GamgLevel &L = g->lev[k], &Ln = g->lev[k + 1];
         int nPadL = L.addr->L.nPad;
         if (c.nPreSweeps)
-            CUDA_TRY(cudaMemcpyAsync(L.pre, L.corr, sizeof(double) * (size_t)L.addr->vecLen, cudaMemcpyDeviceToDevice, st));
-        LAUNCH1D(prolong_kernel, nPadL, st, nPadL, Ln.d_pmap, Ln.corr, L.corr, stop);
+            CUDA_TRY(cudaMemcpyAsync(L.pre.get(), L.corr.get(), sizeof(double) * (size_t)L.addr->vecLen, cudaMemcpyDeviceToDevice, st));
+        LAUNCH1D(prolong_kernel, nPadL, st, nPadL, Ln.d_pmap.get(), Ln.corr.get(), L.corr.get(), stop);
         if (c.interpolateCorrection) {
-            TRY(mat_interpolate(L.mat, L.corr, L.tmp, stop));
+            TRY(mat_interpolate(L.mat.get(), L.corr.get(), L.tmp.get(), stop));
             std::swap(L.corr, L.tmp);
         }
         if (A.scaleCorrection && (c.interpolateCorrection || k < coarsest - 1))
-            TRY(gamg_scale(S, L.mat, L.corr, L.acf, L.src, stop));
+            TRY(gamg_scale(S, L.mat.get(), L.corr.get(), L.acf.get(), L.src.get(), stop));
         if (c.nPreSweeps) {
-            double *corr = L.corr, *pre = L.pre;
+            double *corr = L.corr.get(), *pre = L.pre.get();
             TRY(ew_launch<0>(S.ctx, nPadL / 2, stop, nullptr, nullptr, [=] __device__(int i, double *) {
                 double2 a2 = CV2(corr)[i], p2 = CV2(pre)[i];
                 V2(corr)[i] = make_double2(__dadd_rn(a2.x, p2.x), __dadd_rn(a2.y, p2.y));
             }));
         }
-        TRY(smooth_in_place(S, L.mat, omega, L.corr, L.tmp, L.src,
+        TRY(smooth_in_place(S, L.mat.get(), omega, L.corr, L.tmp, L.src.get(),
                             imin(c.nPostSweeps + c.postSweepsLevelMultiplier * k, c.maxPostSweeps), stop));
     }
     {
         GamgLevel &L0 = g->lev[0];
         int nPadF = fm->a->L.nPad;
-        LAUNCH1D(prolong_kernel, nPadF, st, nPadF, L0.d_pmap, L0.corr, A.finestCorr, stop);
+        LAUNCH1D(prolong_kernel, nPadF, st, nPadF, L0.d_pmap.get(), L0.corr.get(), A.finestCorr, stop);
         KERNEL_CHECK();
     }
     double *psi = A.psiBuf[A.finestSweeps & 1], *spare = A.psiBuf[(A.finestSweeps + 1) & 1];

@@ -5,6 +5,7 @@
 #include <stdio.h>
 #include <string.h>
 
+#include <memory>
 #include <string>
 #include <vector>
 
@@ -34,6 +35,71 @@ void b200_set_error(const char *fmt, ...);
 #define KERNEL_CHECK() CUDA_TRY(cudaGetLastError())
 
 // ---------------------------------------------------------------------------
+// owning buffers: every device (and pinned host) allocation of the library is one of these
+// ---------------------------------------------------------------------------
+// Move-only; the destructor frees.  An empty buffer makes no CUDA call (the host-only layout path needs no
+// GPU).  Never give one static storage duration: it would be freed after the CUDA runtime has shut down.
+template <class T, bool Pinned = false>
+class DevBuf {
+  public:
+    DevBuf() = default;
+    DevBuf(DevBuf &&o) noexcept { std::swap(p_, o.p_), std::swap(n_, o.n_); }
+    DevBuf &operator=(DevBuf &&o) noexcept
+    {
+        if (this != &o) {
+            reset();
+            std::swap(p_, o.p_), std::swap(n_, o.n_);
+        }
+        return *this;
+    }
+    ~DevBuf() { reset(); }
+    T *get() const { return p_; }
+    size_t size() const { return n_; }
+    void reset()
+    {
+        if (p_) Pinned ? cudaFreeHost(p_) : cudaFree(p_);
+        p_ = nullptr, n_ = 0;
+    }
+    // n elements, replacing what was held (contents undefined)
+    int alloc(size_t n)
+    {
+        reset();
+        const size_t bytes = sizeof(T) * n;
+        cudaError_t e = Pinned ? cudaMallocHost((void **)&p_, bytes) : cudaMalloc((void **)&p_, bytes);
+        if (e != cudaSuccess) {
+            p_ = nullptr;
+            b200_set_error("%s of %zu bytes -> %s", Pinned ? "cudaMallocHost" : "cudaMalloc", bytes, cudaGetErrorString(e));
+            return B200LDU_ECUDA;
+        }
+        n_ = n;
+        return B200LDU_OK;
+    }
+    // a copy of h; one element when h is empty
+    int upload(const std::vector<T> &h)
+    {
+        TRY(alloc(h.size() ? h.size() : 1));
+        if (h.size()) CUDA_TRY(cudaMemcpy(p_, h.data(), sizeof(T) * h.size(), cudaMemcpyHostToDevice));
+        return B200LDU_OK;
+    }
+    // at least n elements: never shrinks, does not keep the contents when it reallocates
+    int grow(size_t n) { return p_ && n_ >= n ? B200LDU_OK : alloc(n); }
+
+  private:
+    T *p_ = nullptr;
+    size_t n_ = 0;
+};
+template <class T>
+using PinnedBuf = DevBuf<T, true>;
+
+// an owning handle that is released through its C ABI destroy function (device set, stream synchronised)
+template <class H, int (*Destroy)(H *)>
+struct AbiDestroy {
+    void operator()(H *h) const { Destroy(h); }
+};
+template <class H, int (*Destroy)(H *)>
+using AbiHandle = std::unique_ptr<H, AbiDestroy<H, Destroy>>;
+
+// ---------------------------------------------------------------------------
 // banded layout constants
 // ---------------------------------------------------------------------------
 // A "band" is BAND_ROWS consecutive rows of the renumbered matrix, processed by one
@@ -43,6 +109,24 @@ void b200_set_error(const char *fmt, ...);
 // indices with 32-bit loads (ushort2).
 constexpr int SLICE_ROWS = 64;
 constexpr int ENGINE_THREADS = 256;
+
+// workspace slots (fixed indices: a slot is allocated at its first use and kept)
+enum PoolSlot { POOL_X, POOL_Y, POOL_B, POOL_SLOTS }; // b200ldu_addr::pool, the caller-order matrix operations
+enum WorkSlot {                                        // b200ldu_matrix::work
+    WORK_SOLVER_SLOTS = 8,                             // [0, 8): the vectors of the running solver (Solve::vec)
+    WORK_HOST_PSI = 12, WORK_HOST_SRC,                 // b200ldu_solve_host: caller-order device copies
+    WORK_PSI_B, WORK_SRC_B,                            // b200ldu_solve: banded psi and source
+    WORK_SLOTS
+};
+enum FvmSlot {       // b200ldu_addr::fvmScratch, grown to the largest request
+    FVM_DIAG,        // fvm_solve: boundary-folded diagonal; fvm_residual: boundary-folded source
+    FVM_SOURCE,      // fvm_solve: boundary-folded source, all components
+    FVM_CMPT_SOURCE, // fvm_solve: source of one component
+    FVM_CMPT_PSI,    // fvm_solve: psi of one component; fv_patch_neighbour_field: the send buffer
+    FVM_SLOTS
+};
+
+struct SolverScalars; // ops.cuh
 
 struct b200ldu_ctx {
     int device = 0;
@@ -54,13 +138,12 @@ struct b200ldu_ctx {
     void *nccl = nullptr; // ncclComm_t
     int rank = 0, nRanks = 1;
     // pinned staging for *_host entry points and scalar read-back
-    void *pinned = nullptr;
-    size_t pinnedBytes = 0;
+    PinnedBuf<char> pinned;
     // peer-memory (CUDA IPC over NVLink) collectives, see comm.cu
     bool p2p = false;
-    char *region = nullptr;          // this rank's shared region
+    DevBuf<char> region;             // this rank's shared region
     char *peerRegion[8] = {nullptr}; // every rank's region mapped here (own included)
-    unsigned long long *d_seq = nullptr; // local device counters: [0] reduction seq, [1] halo seq, [2..] scratch
+    DevBuf<unsigned long long> d_seq; // local device counters: [0] reduction seq, [1] halo seq, [2..] scratch
 };
 
 // layout of the IPC-shared region of every rank
@@ -137,38 +220,35 @@ struct b200ldu_addr {
     std::vector<int> perm_h, iperm_h;
     std::vector<double> centres_h; // optional cell centres (kept for GAMG coarse-level banding)
     // device arrays owned
-    long long *d_sliceStart = nullptr;
-    uint16_t *d_sliceW = nullptr, *d_sliceWL = nullptr, *d_col = nullptr;
-    int *d_code = nullptr; // [nEntries] value source: 2f+side | -1 pad | -2-pf interface
-    int *d_haloStart = nullptr, *d_haloIdx = nullptr, *d_perm = nullptr, *d_iperm = nullptr;
-    int *d_sendRows = nullptr; // [nRecv] banded row of faceCells (pack kernel)
-    bool p2pHalo = false;      // peer-store halo usable for this addressing
-    void *d_packPatches = nullptr, *d_packChunks = nullptr; // PackPatch[], PackChunk[] (comm.cu)
+    DevBuf<long long> d_sliceStart;
+    DevBuf<uint16_t> d_sliceW, d_sliceWL, d_col;
+    DevBuf<int> d_code; // [nEntries] value source: 2f+side | -1 pad | -2-pf interface
+    DevBuf<int> d_haloStart, d_haloIdx, d_perm, d_iperm;
+    DevBuf<int> d_sendRows; // [nRecv] banded row of faceCells (pack kernel)
+    bool p2pHalo = false;   // peer-store halo usable for this addressing
+    DevBuf<PackPatch> d_packPatches; // peer-memory halo send descriptors (comm.cu)
+    DevBuf<PackChunk> d_packChunks;
     int nPackChunks = 0;
     double nCellsGlobal = 0;
     // caller-order CSR views for the FV face-sum kernels and faceH
-    int *d_cyclicSrc = nullptr; // per coupled-patch face: banded row supplying it (cyclic partner) | -1
-    int *d_l = nullptr, *d_u = nullptr, *d_ownerStart = nullptr, *d_losort = nullptr,
-        *d_losortStart = nullptr;
+    DevBuf<int> d_cyclicSrc; // per coupled-patch face: banded row supplying it (cyclic partner) | -1
+    DevBuf<int> d_l, d_u, d_ownerStart, d_losort, d_losortStart;
     int nBFaces = 0;
-    int *d_bFaceCells = nullptr;    // boundary faces (all patches, patch order)
-    int *d_bCellStart = nullptr, *d_bCellFaces = nullptr, *d_bCells = nullptr; // per boundary cell lists
-    int nBCells = 0;
+    DevBuf<int> d_bFaceCells;              // boundary faces (all patches, patch order)
+    DevBuf<int> d_bCellStart, d_bCellFaces; // per boundary cell lists
     // fvMatrix glue (fvmatrix.cu): per-cell lists over the coupled patch faces, built at first use, and
     // grow-only scratch vectors
     int nCFaces = 0;
-    int *d_cCellStart = nullptr, *d_cCellFaces = nullptr, *d_cFaceCells = nullptr;
-    double *d_mulesScratch = nullptr; // MULES limiter: six cell fields (mules.cu)
-    size_t mulesScratchLen = 0;
-    double *d_fvmScratch[4] = {nullptr, nullptr, nullptr, nullptr};
-    size_t fvmScratchLen[4] = {0, 0, 0, 0};
+    DevBuf<int> d_cCellStart, d_cCellFaces, d_cFaceCells;
+    DevBuf<double> mulesScratch; // MULES limiter: six cell fields + the received limiters (mules.cu)
+    DevBuf<double> fvmScratch[FVM_SLOTS];
     // host-only structural self-check (b200ldu_layout_debug_*): no GPU, no compute
     bool hostOnly = false;
     std::vector<long long> dbg_sliceStart;
     std::vector<uint16_t> dbg_sliceW, dbg_sliceWL, dbg_col;
     std::vector<int> dbg_code, dbg_haloStart, dbg_haloIdx;
     // workspace pool for caller-order entry points (banded vectors)
-    std::vector<double *> pool;
+    DevBuf<double> pool[POOL_SLOTS];
     long long vecLen = 0; // nPad + nRecv (padded to even)
 };
 
@@ -176,39 +256,29 @@ struct b200ldu_matrix {
     b200ldu_addr *a = nullptr;
     bool symmetric = true;
     bool haveT = false;
-    double *d_val = nullptr;  // banded coefficients for Amul   [nEntries]
-    double *d_valT = nullptr; // banded coefficients for Tmul   (aliases d_val when symmetric)
-    double *d_diag = nullptr; // banded diagonal [nPad] (padding rows = 1)
-    double *d_rD = nullptr;   // 1/diag, filled by matrix_set
+    DevBuf<double> d_val;  // banded coefficients for Amul   [nEntries]
+    DevBuf<double> d_valT; // banded coefficients for Tmul   (only when haveT: A != A^T)
+    DevBuf<double> d_diag; // banded diagonal [nPad] (padding rows = 1)
+    DevBuf<double> d_rD;   // 1/diag, filled by matrix_set
+    const double *valT() const { return haveT ? d_valT.get() : d_val.get(); }
     // caller-order coefficients OWNED by the matrix (copied by matrix_set): diag, upper, lower, interfaceBouCoeffs,
     // interfaceIntCoeffs -- read by faceH, the fvMatrix glue and the GAMG coarse-level assembly
-    double *own[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
-    size_t ownLen[5] = {0, 0, 0, 0, 0};
+    DevBuf<double> own[5];
     // current views of them (diag_ext is re-pointed at the boundary-folded diagonal for the duration of fvm_solve;
     // lower_ext aliases upper_ext when symmetric, int_ext aliases bou_ext when the caller passed one array for both)
     const double *upper_ext = nullptr, *lower_ext = nullptr, *diag_ext = nullptr, *bou_ext = nullptr,
                  *int_ext = nullptr;
     // solver workspace (allocated once, reused across solves -- PCGCache.H:9-58)
-    std::vector<double *> work;
-    double *d_partials = nullptr; // reduction partials
-    void *d_scal = nullptr;       // SolverScalars
-    double *d_hist = nullptr;     // device residual history
-    double *d_sendBuf = nullptr;  // packed psi at coupled-patch face cells
-    int histCap = 0;
+    DevBuf<double> work[WORK_SLOTS];
+    DevBuf<double> d_partials;       // reduction partials
+    DevBuf<SolverScalars> d_scal;
+    DevBuf<double> d_hist;           // device residual history
+    DevBuf<double> d_sendBuf;        // packed psi at coupled-patch face cells
 };
 
 // ---------------------------------------------------------------------------
 // cross-file helpers
 // ---------------------------------------------------------------------------
 int layout_build(b200ldu_addr *a, const double *centres);
-int addr_alloc_vec(b200ldu_addr *a, double **out); // banded vector of vecLen doubles, zeroed
-double *addr_pool_vec(b200ldu_addr *a, int slot);  // reusable scratch (grows on demand)
-
-template <class T>
-int dev_upload(T **d, const std::vector<T> &h)
-{
-    size_t bytes = sizeof(T) * (h.size() ? h.size() : 1);
-    CUDA_TRY(cudaMalloc((void **)d, bytes));
-    if (h.size()) CUDA_TRY(cudaMemcpy(*d, h.data(), sizeof(T) * h.size(), cudaMemcpyHostToDevice));
-    return B200LDU_OK;
-}
+int addr_alloc_vec(b200ldu_addr *a, DevBuf<double> &v); // banded vector of vecLen doubles, zeroed
+double *addr_reuse_vec(b200ldu_addr *a, DevBuf<double> &v); // the same, allocated at first use; null on failure

@@ -425,21 +425,21 @@ int layout_build(b200ldu_addr *a, const double *centres)
     }
 
     // ---- 4. upload ----------------------------------------------------------
-    TRY(dev_upload(&a->d_sliceStart, sliceStart));
-    TRY(dev_upload(&a->d_sliceW, sliceW));
-    TRY(dev_upload(&a->d_sliceWL, sliceWL));
-    TRY(dev_upload(&a->d_col, col));
-    TRY(dev_upload(&a->d_code, code));
-    TRY(dev_upload(&a->d_haloStart, haloStart));
-    TRY(dev_upload(&a->d_haloIdx, haloIdx));
-    TRY(dev_upload(&a->d_perm, a->perm_h));
-    TRY(dev_upload(&a->d_iperm, a->iperm_h));
-    TRY(dev_upload(&a->d_sendRows, sendRows));
-    TRY(dev_upload(&a->d_l, a->l));
-    TRY(dev_upload(&a->d_u, a->u));
-    TRY(dev_upload(&a->d_ownerStart, ownerStart));
-    TRY(dev_upload(&a->d_losort, losort));
-    TRY(dev_upload(&a->d_losortStart, losortStart));
+    TRY(a->d_sliceStart.upload(sliceStart));
+    TRY(a->d_sliceW.upload(sliceW));
+    TRY(a->d_sliceWL.upload(sliceWL));
+    TRY(a->d_col.upload(col));
+    TRY(a->d_code.upload(code));
+    TRY(a->d_haloStart.upload(haloStart));
+    TRY(a->d_haloIdx.upload(haloIdx));
+    TRY(a->d_perm.upload(a->perm_h));
+    TRY(a->d_iperm.upload(a->iperm_h));
+    TRY(a->d_sendRows.upload(sendRows));
+    TRY(a->d_l.upload(a->l));
+    TRY(a->d_u.upload(a->u));
+    TRY(a->d_ownerStart.upload(ownerStart));
+    TRY(a->d_losort.upload(losort));
+    TRY(a->d_losortStart.upload(losortStart));
 
     LayoutDev &L = a->L;
     L.nCells = nCells;
@@ -449,14 +449,14 @@ int layout_build(b200ldu_addr *a, const double *centres)
     L.slicesPerBand = slicesPerBand;
     L.nRecv = nRecv;
     L.maxHalo = maxHalo;
-    L.sliceStart = a->d_sliceStart;
-    L.sliceW = a->d_sliceW;
-    L.sliceWL = a->d_sliceWL;
-    L.col = a->d_col;
-    L.haloStart = a->d_haloStart;
-    L.haloIdx = a->d_haloIdx;
-    L.perm = a->d_perm;
-    L.iperm = a->d_iperm;
+    L.sliceStart = a->d_sliceStart.get();
+    L.sliceW = a->d_sliceW.get();
+    L.sliceWL = a->d_sliceWL.get();
+    L.col = a->d_col.get();
+    L.haloStart = a->d_haloStart.get();
+    L.haloIdx = a->d_haloIdx.get();
+    L.perm = a->d_perm.get();
+    L.iperm = a->d_iperm.get();
     a->nEntries = nEntries;
     a->nHaloTotal = haloStart[nBands];
     a->vecLen = ((long long)nPad + nRecv + 1) & ~1ll;
@@ -472,7 +472,7 @@ extern "C" int b200ldu_layout_debug_create(int nCells, int nFaces, const int *lo
                                            const double *cellCentres_h, b200ldu_addr **out)
 {
     if (!out || nCells <= 0) return B200LDU_EINVAL;
-    b200ldu_addr *a = new b200ldu_addr();
+    std::unique_ptr<b200ldu_addr> a(new b200ldu_addr()); // plain delete: no CUDA call on this path
     a->hostOnly = true;
     a->nCells = nCells;
     a->nFaces = nFaces;
@@ -483,12 +483,8 @@ extern "C" int b200ldu_layout_debug_create(int nCells, int nFaces, const int *lo
         a->patchStart.assign(patchStart_h, patchStart_h + nPatches + 1);
         a->faceCells.assign(faceCells_h, faceCells_h + a->patchStart[nPatches]);
     }
-    int rc = layout_build(a, cellCentres_h);
-    if (rc != B200LDU_OK) {
-        delete a;
-        return rc;
-    }
-    *out = a;
+    TRY(layout_build(a.get(), cellCentres_h));
+    *out = a.release();
     return B200LDU_OK;
 }
 

@@ -65,16 +65,15 @@ extern "C" int b200ldu_ctx_create(int device, b200ldu_ctx **out)
         return B200LDU_EINVAL;
     }
     CUDA_TRY(cudaSetDevice(device));
-    b200ldu_ctx *c = new b200ldu_ctx();
+    AbiHandle<b200ldu_ctx, b200ldu_ctx_destroy> c(new b200ldu_ctx());
     c->device = device;
     cudaDeviceProp p;
     CUDA_TRY(cudaGetDeviceProperties(&p, device));
     c->smCount = p.multiProcessorCount;
     CUDA_TRY(cudaStreamCreateWithFlags(&c->ownStream, cudaStreamNonBlocking));
     c->stream = c->ownStream;
-    c->pinnedBytes = 1 << 16;
-    CUDA_TRY(cudaMallocHost(&c->pinned, c->pinnedBytes));
-    *out = c;
+    TRY(c->pinned.alloc(1 << 16));
+    *out = c.release();
     return B200LDU_OK;
 }
 
@@ -84,7 +83,6 @@ extern "C" int b200ldu_ctx_destroy(b200ldu_ctx *c)
     cudaSetDevice(c->device);
     cudaStreamSynchronize(c->stream);
     comm_destroy(c);
-    if (c->pinned) cudaFreeHost(c->pinned);
     if (c->ownStream) cudaStreamDestroy(c->ownStream);
     delete c;
     return B200LDU_OK;
@@ -105,19 +103,6 @@ extern "C" int b200ldu_ctx_sync(b200ldu_ctx *c)
 
 extern "C" long long b200ldu_launch_count(const b200ldu_ctx *c) { return c ? c->launches : 0; }
 
-int ctx_pinned(b200ldu_ctx *c, size_t bytes, void **out)
-{
-    if (bytes > c->pinnedBytes) {
-        if (c->pinned) cudaFreeHost(c->pinned);
-        c->pinned = nullptr;
-        c->pinnedBytes = 0;
-        CUDA_TRY(cudaMallocHost(&c->pinned, bytes));
-        c->pinnedBytes = bytes;
-    }
-    *out = c->pinned;
-    return B200LDU_OK;
-}
-
 // ---------------------------------------------------------------------------
 // addressing
 // ---------------------------------------------------------------------------
@@ -132,7 +117,7 @@ extern "C" int b200ldu_addr_create(b200ldu_ctx *ctx, int nCells, int nFaces, con
         return B200LDU_EINVAL;
     }
     CUDA_TRY(cudaSetDevice(ctx->device));
-    b200ldu_addr *a = new b200ldu_addr();
+    AbiHandle<b200ldu_addr, b200ldu_addr_destroy> a(new b200ldu_addr());
     a->ctx = ctx;
     a->nCells = nCells;
     a->nFaces = nFaces;
@@ -146,21 +131,12 @@ extern "C" int b200ldu_addr_create(b200ldu_ctx *ctx, int nCells, int nFaces, con
         for (int i = 0; i < a->patchStart[nPatches]; i++)
             if (a->faceCells[i] < 0 || a->faceCells[i] >= nCells) {
                 b200_set_error("addr_create: patch faceCells out of range");
-                delete a;
                 return B200LDU_EINVAL;
             }
     }
     if (cellCentres_h) a->centres_h.assign(cellCentres_h, cellCentres_h + 3 * (size_t)nCells);
-    int rc = layout_build(a, cellCentres_h);
-    if (rc != B200LDU_OK) {
-        b200ldu_addr_destroy(a);
-        return rc;
-    }
-    rc = comm_addr_setup(a);
-    if (rc != B200LDU_OK) {
-        b200ldu_addr_destroy(a);
-        return rc;
-    }
+    TRY(layout_build(a.get(), cellCentres_h));
+    TRY(comm_addr_setup(a.get()));
     // cyclic patches: neighbRank[p] = -(q+1) pairs patch p with patch q of this addressing, face i
     // with face i (cyclicLduInterface: neighbPatchID).  Their "received" values are psi at the
     // partner's face cells, copied on the device (comm_halo_exchange).
@@ -176,21 +152,15 @@ extern "C" int b200ldu_addr_create(b200ldu_ctx *ctx, int nCells, int nFaces, con
                 if (q < 0 || q >= nPatches || q == p || a->neighbRank[q] != -(p + 1) ||
                     a->patchStart[q + 1] - a->patchStart[q] != n) {
                     b200_set_error("addr_create: cyclic patch %d has no matching partner patch", p);
-                    b200ldu_addr_destroy(a);
                     return B200LDU_EINVAL;
                 }
                 for (int i = 0; i < n; i++)
                     src[(size_t)a->patchStart[p] + i] = a->perm_h[a->faceCells[(size_t)a->patchStart[q] + i]];
             }
-            if (cudaMalloc((void **)&a->d_cyclicSrc, sizeof(int) * src.size()) != cudaSuccess ||
-                cudaMemcpy(a->d_cyclicSrc, src.data(), sizeof(int) * src.size(), cudaMemcpyHostToDevice) != cudaSuccess) {
-                b200_set_error("addr_create: out of device memory");
-                b200ldu_addr_destroy(a);
-                return B200LDU_ECUDA;
-            }
+            TRY(a->d_cyclicSrc.upload(src));
         }
     }
-    *out = a;
+    *out = a.release();
     return B200LDU_OK;
 }
 
@@ -199,16 +169,6 @@ extern "C" int b200ldu_addr_destroy(b200ldu_addr *a)
     if (!a) return B200LDU_OK;
     cudaSetDevice(a->ctx->device);
     cudaStreamSynchronize(a->ctx->stream);
-    void *ptrs[] = {a->d_sliceStart, a->d_sliceW, a->d_sliceWL, a->d_col, a->d_code, a->d_haloStart,
-                    a->d_haloIdx, a->d_perm, a->d_iperm, a->d_sendRows, a->d_l, a->d_u,
-                    a->d_ownerStart, a->d_losort, a->d_losortStart, a->d_bFaceCells, a->d_cyclicSrc,
-                    a->d_bCellStart, a->d_bCellFaces, a->d_bCells, a->d_packPatches, a->d_packChunks,
-                    a->d_cCellStart, a->d_cCellFaces, a->d_cFaceCells, a->d_mulesScratch, a->d_fvmScratch[0],
-                    a->d_fvmScratch[1], a->d_fvmScratch[2], a->d_fvmScratch[3]};
-    for (void *p : ptrs)
-        if (p) cudaFree(p);
-    for (double *p : a->pool)
-        if (p) cudaFree(p);
     delete a;
     return B200LDU_OK;
 }
@@ -234,21 +194,20 @@ extern "C" int b200ldu_addr_perm(const b200ldu_addr *a, int *perm_h)
 
 extern "C" long long b200ldu_vec_len(const b200ldu_addr *a) { return a ? a->vecLen : 0; }
 
-int addr_alloc_vec(b200ldu_addr *a, double **out)
+int addr_alloc_vec(b200ldu_addr *a, DevBuf<double> &v)
 {
-    CUDA_TRY(cudaMalloc((void **)out, sizeof(double) * (size_t)a->vecLen));
-    CUDA_TRY(cudaMemsetAsync(*out, 0, sizeof(double) * (size_t)a->vecLen, a->ctx->stream));
+    TRY(v.alloc((size_t)a->vecLen));
+    CUDA_TRY(cudaMemsetAsync(v.get(), 0, sizeof(double) * (size_t)a->vecLen, a->ctx->stream));
     return B200LDU_OK;
 }
 
-double *addr_pool_vec(b200ldu_addr *a, int slot)
+double *addr_reuse_vec(b200ldu_addr *a, DevBuf<double> &v)
 {
-    while ((int)a->pool.size() <= slot) a->pool.push_back(nullptr);
-    if (!a->pool[slot]) {
-        if (addr_alloc_vec(a, &a->pool[slot]) != B200LDU_OK) return nullptr;
-    }
-    return a->pool[slot];
+    if (!v.get() && addr_alloc_vec(a, v) != B200LDU_OK) return nullptr;
+    return v.get();
 }
+
+static double *addr_pool_vec(b200ldu_addr *a, PoolSlot slot) { return addr_reuse_vec(a, a->pool[slot]); }
 
 // ---- caller order <-> banded order ----
 __global__ void to_banded_kernel(int nPad, const int *__restrict__ iperm, const double *__restrict__ x,
@@ -270,7 +229,7 @@ __global__ void from_banded_kernel(int nCells, const int *__restrict__ iperm,
 
 int to_banded(b200ldu_addr *a, const double *x, double *xb)
 {
-    to_banded_kernel<<<(a->L.nPad + 255) / 256, 256, 0, a->ctx->stream>>>(a->L.nPad, a->d_iperm, x, xb);
+    to_banded_kernel<<<(a->L.nPad + 255) / 256, 256, 0, a->ctx->stream>>>(a->L.nPad, a->d_iperm.get(), x, xb);
     a->ctx->launches++;
     KERNEL_CHECK();
     return B200LDU_OK;
@@ -279,7 +238,7 @@ int to_banded(b200ldu_addr *a, const double *x, double *xb)
 int from_banded(b200ldu_addr *a, const double *xb, double *x)
 {
     // rows [0, nCells) are the real rows (padding sits at the end)
-    from_banded_kernel<<<(a->nCells + 255) / 256, 256, 0, a->ctx->stream>>>(a->nCells, a->d_iperm, xb, x);
+    from_banded_kernel<<<(a->nCells + 255) / 256, 256, 0, a->ctx->stream>>>(a->nCells, a->d_iperm.get(), xb, x);
     a->ctx->launches++;
     KERNEL_CHECK();
     return B200LDU_OK;
@@ -304,17 +263,17 @@ extern "C" int b200ldu_matrix_create(b200ldu_addr *a, b200ldu_matrix **out)
 {
     if (!a || !out) return B200LDU_EINVAL;
     CUDA_TRY(cudaSetDevice(a->ctx->device));
-    b200ldu_matrix *m = new b200ldu_matrix();
+    AbiHandle<b200ldu_matrix, b200ldu_matrix_destroy> m(new b200ldu_matrix());
     m->a = a;
     // coefficient streams are allocated by matrix_set (which layout is used depends on symmetry)
-    CUDA_TRY(cudaMalloc((void **)&m->d_diag, sizeof(double) * (size_t)a->vecLen));
-    CUDA_TRY(cudaMalloc((void **)&m->d_rD, sizeof(double) * (size_t)a->vecLen));
+    TRY(m->d_diag.alloc((size_t)a->vecLen));
+    TRY(m->d_rD.alloc((size_t)a->vecLen));
     int np = a->L.nBands > a->ctx->smCount * 8 ? a->L.nBands : a->ctx->smCount * 8;
-    CUDA_TRY(cudaMalloc((void **)&m->d_partials, sizeof(double) * 4 * (size_t)np));
-    CUDA_TRY(cudaMalloc((void **)&m->d_scal, sizeof(SolverScalars)));
-    CUDA_TRY(cudaMemset(m->d_scal, 0, sizeof(SolverScalars)));
-    CUDA_TRY(cudaMalloc((void **)&m->d_sendBuf, sizeof(double) * (size_t)(a->L.nRecv > 0 ? a->L.nRecv : 1)));
-    *out = m;
+    TRY(m->d_partials.alloc(4 * (size_t)np));
+    TRY(m->d_scal.alloc(1));
+    CUDA_TRY(cudaMemset(m->d_scal.get(), 0, sizeof(SolverScalars)));
+    TRY(m->d_sendBuf.alloc((size_t)(a->L.nRecv > 0 ? a->L.nRecv : 1)));
+    *out = m.release();
     return B200LDU_OK;
 }
 
@@ -323,13 +282,6 @@ extern "C" int b200ldu_matrix_destroy(b200ldu_matrix *m)
     if (!m) return B200LDU_OK;
     cudaSetDevice(m->a->ctx->device);
     cudaStreamSynchronize(m->a->ctx->stream);
-    if (m->d_valT && m->d_valT != m->d_val) cudaFree(m->d_valT);
-    void *ptrs[] = {m->d_val, m->d_diag, m->d_rD, m->d_partials, m->d_scal, m->d_hist, m->d_sendBuf,
-                    m->own[0], m->own[1], m->own[2], m->own[3], m->own[4]};
-    for (void *p : ptrs)
-        if (p) cudaFree(p);
-    for (double *p : m->work)
-        if (p) cudaFree(p);
     delete m;
     return B200LDU_OK;
 }
@@ -378,16 +330,10 @@ static int own_copy(b200ldu_matrix *m, int k, const double *src, size_t n, const
 {
     *out = nullptr;
     if (!src || n == 0) return B200LDU_OK;
-    if (m->ownLen[k] < n) {
-        if (m->own[k]) cudaFree(m->own[k]);
-        m->own[k] = nullptr;
-        m->ownLen[k] = 0;
-        CUDA_TRY(cudaMalloc((void **)&m->own[k], sizeof(double) * n));
-        m->ownLen[k] = n;
-    }
-    if (src != m->own[k])
-        CUDA_TRY(cudaMemcpyAsync(m->own[k], src, sizeof(double) * n, cudaMemcpyDeviceToDevice, m->a->ctx->stream));
-    *out = m->own[k];
+    TRY(m->own[k].grow(n));
+    if (src != m->own[k].get())
+        CUDA_TRY(cudaMemcpyAsync(m->own[k].get(), src, sizeof(double) * n, cudaMemcpyDeviceToDevice, m->a->ctx->stream));
+    *out = m->own[k].get();
     return B200LDU_OK;
 }
 
@@ -396,8 +342,8 @@ static int own_copy(b200ldu_matrix *m, int k, const double *src, size_t n, const
 int matrix_set_diag(b200ldu_matrix *m, const double *diag_d)
 {
     b200ldu_addr *a = m->a;
-    fill_diag_kernel<<<(unsigned)((a->vecLen + 255) / 256), 256, 0, a->ctx->stream>>>(a->vecLen, a->L.nPad, a->d_iperm,
-                                                                                      diag_d, m->d_diag, m->d_rD);
+    fill_diag_kernel<<<(unsigned)((a->vecLen + 255) / 256), 256, 0, a->ctx->stream>>>(a->vecLen, a->L.nPad, a->d_iperm.get(),
+                                                                                      diag_d, m->d_diag.get(), m->d_rD.get());
     a->ctx->launches++;
     KERNEL_CHECK();
     m->diag_ext = diag_d;
@@ -437,27 +383,23 @@ extern "C" int b200ldu_matrix_set(b200ldu_matrix *m, const double *diag_d, const
     // Tmul needs its own coefficient stream when A != A^T (asymmetric coefficients or
     // interfaceIntCoeffs != interfaceBouCoeffs)
     bool needT = !m->symmetric || (a->L.nRecv && !sameIfc);
-    size_t nb = sizeof(double) * (size_t)(ne > 0 ? ne : 1);
-    if (!m->d_val) CUDA_TRY(cudaMalloc((void **)&m->d_val, nb));
-    if (needT && (!m->d_valT || m->d_valT == m->d_val)) {
-        m->d_valT = nullptr;
-        CUDA_TRY(cudaMalloc((void **)&m->d_valT, nb));
-    }
+    size_t nb = (size_t)(ne > 0 ? ne : 1);
+    if (!m->d_val.get()) TRY(m->d_val.alloc(nb));
+    if (!needT)
+        m->d_valT.reset(); // A^T == A
+    else if (!m->d_valT.get())
+        TRY(m->d_valT.alloc(nb));
+    m->haveT = needT;
     if (ne > 0) {
         unsigned g = (unsigned)((ne + 255) / 256);
-        fill_val_kernel<<<g, 256, 0, st>>>(ne, a->d_code, up, lo, bo, m->d_val, 0);
+        fill_val_kernel<<<g, 256, 0, st>>>(ne, a->d_code.get(), up, lo, bo, m->d_val.get(), 0);
         a->ctx->launches++;
         if (needT) {
-            fill_val_kernel<<<g, 256, 0, st>>>(ne, a->d_code, up, lo, in, m->d_valT, 1);
+            fill_val_kernel<<<g, 256, 0, st>>>(ne, a->d_code.get(), up, lo, in, m->d_valT.get(), 1);
             a->ctx->launches++;
         }
     }
-    if (!needT) {
-        if (m->d_valT && m->d_valT != m->d_val) cudaFree(m->d_valT);
-        m->d_valT = m->d_val; // A^T == A
-    }
     KERNEL_CHECK();
-    m->haveT = needT;
     m->upper_ext = up;
     m->bou_ext = bo;
     m->int_ext = in;
@@ -470,7 +412,7 @@ extern "C" int b200ldu_matrix_set(b200ldu_matrix *m, const double *diag_d, const
 // ---------------------------------------------------------------------------
 int mat_halo(b200ldu_matrix *m, double *x, const int *stop, int *usedP2P)
 {
-    return comm_halo_exchange(m->a, x, m->d_sendBuf, stop, usedP2P);
+    return comm_halo_exchange(m->a, x, m->d_sendBuf.get(), stop, usedP2P);
 }
 
 int mat_amul(b200ldu_matrix *m, bool transpose, double *x, double *out, int mode, const double *aux,
@@ -485,7 +427,7 @@ int mat_amul(b200ldu_matrix *m, bool transpose, double *x, double *out, int mode
         op.waitHalo = wait;                \
         op.partials = partials;            \
         op.x = x;                          \
-        op.diag = m->d_diag;               \
+        op.diag = m->d_diag.get();         \
         op.aux = aux;                      \
         op.out = out;                      \
         return engine_launch_m(m, transpose, op); \
@@ -509,7 +451,7 @@ int mat_ainv(b200ldu_matrix *m, bool transpose, const double *r, double *w, bool
         op.stop = stop;
         op.partials = partials;
         op.r = r;
-        op.rD = m->d_rD;
+        op.rD = m->d_rD.get();
         op.dotv = dotv;
         op.out = w;
         return engine_launch_m(m, transpose, op);
@@ -518,7 +460,7 @@ int mat_ainv(b200ldu_matrix *m, bool transpose, const double *r, double *w, bool
     op.stop = stop;
     op.partials = partials;
     op.r = r;
-    op.rD = m->d_rD;
+    op.rD = m->d_rD.get();
     op.dotv = nullptr;
     op.out = w;
     return engine_launch_m(m, transpose, op);
@@ -532,7 +474,7 @@ int mat_jacobi(b200ldu_matrix *m, double omega, double *x, const double *b, doub
     op.stop = stop;
     op.waitHalo = wait;
     op.x = x;
-    op.diag = m->d_diag;
+    op.diag = m->d_diag.get();
     op.b = b;
     op.out = out;
     op.omega = omega;
@@ -551,7 +493,7 @@ int mat_residual(b200ldu_matrix *m, double *x, const double *b, double *out, boo
         op.waitHalo = wait;
         op.partials = partials;
         op.x = x;
-        op.diag = m->d_diag;
+        op.diag = m->d_diag.get();
         op.b = b;
         op.out = out;
         return engine_launch_m(m, false, op);
@@ -560,7 +502,7 @@ int mat_residual(b200ldu_matrix *m, double *x, const double *b, double *out, boo
     op.stop = stop;
     op.waitHalo = wait;
     op.x = x;
-    op.diag = m->d_diag;
+    op.diag = m->d_diag.get();
     op.b = b;
     op.out = out;
     return engine_launch_m(m, false, op);
@@ -570,7 +512,7 @@ int mat_sumA(b200ldu_matrix *m, double *out, const int *stop)
 {
     CoeffSumOp<false, false> op;
     op.stop = stop;
-    op.diag = m->d_diag;
+    op.diag = m->d_diag.get();
     op.out = out;
     return engine_launch_m(m, false, op);
 }
@@ -587,7 +529,7 @@ int mat_H(b200ldu_matrix *m, const double *x, double *out)
 {
     OffDiagOp<true, false> op;
     op.x = x;
-    op.diag = m->d_diag;
+    op.diag = m->d_diag.get();
     op.out = out;
     return engine_launch_m(m, false, op);
 }
@@ -600,7 +542,7 @@ int mat_interpolate(b200ldu_matrix *m, double *x, double *out, const int *stop)
     op.stop = stop;
     op.waitHalo = wait;
     op.x = x;
-    op.diag = m->d_diag;
+    op.diag = m->d_diag.get();
     op.out = out;
     return engine_launch_m(m, false, op);
 }
@@ -620,7 +562,7 @@ static int amul_ext(b200ldu_matrix *m, bool T, const double *psi, double *out)
     CHECK_M(m);
     if (!psi || !out) return B200LDU_EINVAL;
     b200ldu_addr *a = m->a;
-    double *xb = addr_pool_vec(a, 0), *yb = addr_pool_vec(a, 1);
+    double *xb = addr_pool_vec(a, POOL_X), *yb = addr_pool_vec(a, POOL_Y);
     if (!xb || !yb) return B200LDU_ECUDA;
     TRY(to_banded(a, psi, xb));
     TRY(mat_amul(m, T, xb, yb, 0, nullptr, nullptr, nullptr));
@@ -646,7 +588,7 @@ extern "C" int b200ldu_amul_banded(b200ldu_matrix *m, const double *psib_d, doub
 extern "C" int b200ldu_sumA(b200ldu_matrix *m, double *sumA_d)
 {
     CHECK_M(m);
-    double *yb = addr_pool_vec(m->a, 1);
+    double *yb = addr_pool_vec(m->a, POOL_Y);
     if (!yb) return B200LDU_ECUDA;
     TRY(mat_sumA(m, yb, nullptr));
     return from_banded(m->a, yb, sumA_d);
@@ -657,7 +599,7 @@ extern "C" int b200ldu_residual(b200ldu_matrix *m, const double *psi_d, const do
 {
     CHECK_M(m);
     b200ldu_addr *a = m->a;
-    double *xb = addr_pool_vec(a, 0), *yb = addr_pool_vec(a, 1), *bb = addr_pool_vec(a, 2);
+    double *xb = addr_pool_vec(a, POOL_X), *yb = addr_pool_vec(a, POOL_Y), *bb = addr_pool_vec(a, POOL_B);
     if (!xb || !yb || !bb) return B200LDU_ECUDA;
     TRY(to_banded(a, psi_d, xb));
     TRY(to_banded(a, source_d, bb));
@@ -669,7 +611,7 @@ extern "C" int b200ldu_H(b200ldu_matrix *m, const double *psi_d, double *Hpsi_d)
 {
     CHECK_M(m);
     b200ldu_addr *a = m->a;
-    double *xb = addr_pool_vec(a, 0), *yb = addr_pool_vec(a, 1);
+    double *xb = addr_pool_vec(a, POOL_X), *yb = addr_pool_vec(a, POOL_Y);
     if (!xb || !yb) return B200LDU_ECUDA;
     TRY(to_banded(a, psi_d, xb));
     TRY(mat_H(m, xb, yb));
@@ -679,7 +621,7 @@ extern "C" int b200ldu_H(b200ldu_matrix *m, const double *psi_d, double *Hpsi_d)
 extern "C" int b200ldu_H1(b200ldu_matrix *m, double *H1_d)
 {
     CHECK_M(m);
-    double *yb = addr_pool_vec(m->a, 1);
+    double *yb = addr_pool_vec(m->a, POOL_Y);
     if (!yb) return B200LDU_ECUDA;
     TRY(mat_H1(m, yb));
     return from_banded(m->a, yb, H1_d);
@@ -704,7 +646,7 @@ extern "C" int b200ldu_faceH(b200ldu_matrix *m, const double *psi_d, double *fac
         return B200LDU_EINVAL;
     }
     if (a->nFaces == 0) return B200LDU_OK;
-    faceH_kernel<<<(a->nFaces + 255) / 256, 256, 0, a->ctx->stream>>>(a->nFaces, a->d_l, a->d_u, m->upper_ext,
+    faceH_kernel<<<(a->nFaces + 255) / 256, 256, 0, a->ctx->stream>>>(a->nFaces, a->d_l.get(), a->d_u.get(), m->upper_ext,
                                                                         m->lower_ext, psi_d, faceHpsi_d);
     a->ctx->launches++;
     KERNEL_CHECK();
@@ -738,7 +680,7 @@ int mat_precondition(b200ldu_matrix *m, int kind, bool transpose, const double *
         if (nPartials) *nPartials = a->L.nBands;
         return mat_ainv(m, transpose, r, w, fuseDot, dotv, partials, stop);
     }
-    const double *rD = m->d_rD;
+    const double *rD = m->d_rD.get();
     const double *dv = dotv ? dotv : r;
     int n2 = a->L.nPad / 2;
     if (kind == 1) { // diagonalPreconditioner.C:76-89
@@ -778,7 +720,7 @@ extern "C" int b200ldu_precondition(b200ldu_matrix *m, const char *name, int tra
     int k = precond_kind(name, printed);
     if (k < 0) return B200LDU_ENOPRECOND;
     b200ldu_addr *a = m->a;
-    double *xb = addr_pool_vec(a, 0), *yb = addr_pool_vec(a, 1);
+    double *xb = addr_pool_vec(a, POOL_X), *yb = addr_pool_vec(a, POOL_Y);
     if (!xb || !yb) return B200LDU_ECUDA;
     TRY(to_banded(a, rA_d, xb));
     TRY(mat_precondition(m, k, transpose != 0, xb, yb, false, nullptr, nullptr, nullptr, nullptr));
@@ -799,7 +741,7 @@ extern "C" int b200ldu_smooth(b200ldu_matrix *m, const char *name, double omega,
     CHECK_M(m);
     if (!smoother_ok(name)) return B200LDU_ENOPRECOND;
     b200ldu_addr *a = m->a;
-    double *xb = addr_pool_vec(a, 0), *yb = addr_pool_vec(a, 1), *bb = addr_pool_vec(a, 2);
+    double *xb = addr_pool_vec(a, POOL_X), *yb = addr_pool_vec(a, POOL_Y), *bb = addr_pool_vec(a, POOL_B);
     if (!xb || !yb || !bb) return B200LDU_ECUDA;
     TRY(to_banded(a, psi_d, xb));
     TRY(to_banded(a, source_d, bb));
@@ -821,11 +763,11 @@ extern "C" int b200ldu_bench_op(b200ldu_matrix *m, const char *op, double *xb, d
     if (!op || !xb || !yb) return B200LDU_EINVAL;
     if (!strcmp(op, "amul")) return mat_amul(m, false, xb, yb, 0, nullptr, nullptr, nullptr);
     if (!strcmp(op, "tmul")) return mat_amul(m, true, xb, yb, 0, nullptr, nullptr, nullptr);
-    if (!strcmp(op, "amul_dot")) return mat_amul(m, false, xb, yb, 1, nullptr, m->d_partials, nullptr);
+    if (!strcmp(op, "amul_dot")) return mat_amul(m, false, xb, yb, 1, nullptr, m->d_partials.get(), nullptr);
     if (!strcmp(op, "ainv")) return mat_ainv(m, false, xb, yb, false, nullptr, nullptr, nullptr);
-    if (!strcmp(op, "ainv_dot")) return mat_ainv(m, false, xb, yb, true, nullptr, m->d_partials, nullptr);
+    if (!strcmp(op, "ainv_dot")) return mat_ainv(m, false, xb, yb, true, nullptr, m->d_partials.get(), nullptr);
     if (!strcmp(op, "jacobi")) return bb ? mat_jacobi(m, 0.9, xb, bb, yb, nullptr) : B200LDU_EINVAL;
-    if (!strcmp(op, "residual")) return bb ? mat_residual(m, xb, bb, yb, true, m->d_partials, nullptr) : B200LDU_EINVAL;
+    if (!strcmp(op, "residual")) return bb ? mat_residual(m, xb, bb, yb, true, m->d_partials.get(), nullptr) : B200LDU_EINVAL;
     if (!strcmp(op, "sumA")) return mat_sumA(m, yb, nullptr);
     if (!strcmp(op, "H")) return mat_H(m, xb, yb);
     b200_set_error("bench_op: unknown op %s", op);

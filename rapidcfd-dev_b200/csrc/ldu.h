@@ -2,7 +2,6 @@
 #pragma once
 #include "internal.h"
 
-int ctx_pinned(b200ldu_ctx *c, size_t bytes, void **out);
 int matrix_set_diag(b200ldu_matrix *m, const double *diag_d); // banded diag + 1/diag; re-points diag_ext
 int to_banded(b200ldu_addr *a, const double *x, double *xb);
 int from_banded(b200ldu_addr *a, const double *xb, double *x);

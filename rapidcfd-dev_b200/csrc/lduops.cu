@@ -66,8 +66,8 @@ extern "C" int b200ldu_ldu_row_sum(b200ldu_addr *a, int mode, const double *uppe
 {
     if (!a || !inout_d || mode < 0 || mode > 2 || (a->nFaces && !upper_d)) return B200LDU_EINVAL;
     CUDA_TRY(cudaSetDevice(a->ctx->device));
-    row_sum_kernel<<<(a->nCells + 127) / 128, 128, 0, a->ctx->stream>>>(a->nCells, mode, a->d_ownerStart, a->d_losortStart,
-                                                                        a->d_losort, upper_d, lower_d ? lower_d : upper_d, inout_d);
+    row_sum_kernel<<<(a->nCells + 127) / 128, 128, 0, a->ctx->stream>>>(a->nCells, mode, a->d_ownerStart.get(), a->d_losortStart.get(),
+                                                                        a->d_losort.get(), upper_d, lower_d ? lower_d : upper_d, inout_d);
     a->ctx->launches++;
     KERNEL_CHECK();
     return B200LDU_OK;
@@ -132,8 +132,8 @@ extern "C" int b200ldu_ldu_scale(b200ldu_addr *a, const double *sf_d, double s, 
     CUDA_TRY(cudaSetDevice(ctx->device));
     const long long n = a->nCells, nF = a->nFaces;
     if (hasA[0] && diagA_d && n) scale_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(n, nullptr, sf_d, s, diagA_d);
-    if (hasA[1] && upperA_d && nF) scale_kernel<<<(unsigned)((nF + 255) / 256), 256, 0, ctx->stream>>>(nF, a->d_l, sf_d, s, upperA_d);
-    if (hasA[2] && lowerA_d && nF) scale_kernel<<<(unsigned)((nF + 255) / 256), 256, 0, ctx->stream>>>(nF, a->d_u, sf_d, s, lowerA_d);
+    if (hasA[1] && upperA_d && nF) scale_kernel<<<(unsigned)((nF + 255) / 256), 256, 0, ctx->stream>>>(nF, a->d_l.get(), sf_d, s, upperA_d);
+    if (hasA[2] && lowerA_d && nF) scale_kernel<<<(unsigned)((nF + 255) / 256), 256, 0, ctx->stream>>>(nF, a->d_u.get(), sf_d, s, lowerA_d);
     ctx->launches += 3;
     KERNEL_CHECK();
     return B200LDU_OK;

@@ -33,27 +33,21 @@ static int mules_limiter_impl(int corr, double extrema, b200ldu_addr *a, int nLi
     const int n = a->nCells, nF = a->nFaces, nB = a->nBFaces;
     // scratch: psiMaxn, psiMinn, sumPhip, mSumPhim, lambdam, lambdap (six cell fields, kept across calls) + the received limiters
     const size_t need = (size_t)6 * n + (size_t)nCoupledFaces;
-    if (a->mulesScratchLen < need) {
-        if (a->d_mulesScratch) cudaFree(a->d_mulesScratch);
-        a->d_mulesScratch = nullptr;
-        a->mulesScratchLen = 0;
-        CUDA_TRY(cudaMalloc((void **)&a->d_mulesScratch, sizeof(double) * need));
-        a->mulesScratchLen = need;
-    }
-    double *psiMaxn = a->d_mulesScratch, *psiMinn = psiMaxn + n, *sumPhip = psiMinn + n, *mSumPhim = sumPhip + n,
+    TRY(a->mulesScratch.grow(need));
+    double *psiMaxn = a->mulesScratch.get(), *psiMinn = psiMaxn + n, *sumPhip = psiMinn + n, *mSumPhim = sumPhip + n,
            *lambdam = mSumPhim + n, *lambdap = lambdam + n, *theirs = lambdap + n;
-    const int *bs = nB ? a->d_bCellStart : nullptr;
+    const int *bs = nB ? a->d_bCellStart.get() : nullptr;
     // lambda_d / lambdaB_d come in holding the starting limiter (MULES::limit: allLambda(mesh.nFaces(), 1.0))
-    mules_bounds_kernel<<<(n + 127) / 128, 128, 0, st>>>(n, a->d_ownerStart, a->d_u, a->d_losortStart, a->d_losort, a->d_l, bs,
-                                                         a->d_bCellFaces, psi_d, psiB_d, phiBD_d, phiBDB_d, phiCorr_d, phiCorrB_d,
+    mules_bounds_kernel<<<(n + 127) / 128, 128, 0, st>>>(n, a->d_ownerStart.get(), a->d_u.get(), a->d_losortStart.get(), a->d_losort.get(), a->d_l.get(), bs,
+                                                         a->d_bCellFaces.get(), psi_d, psiB_d, phiBD_d, phiBDB_d, phiCorr_d, phiCorrB_d,
                                                          psi0_d, rho_d, rho0_d, Sp_d, Su_d, V_d, rDeltaT, psiMax, psiMin, psiMaxn,
                                                          psiMinn, sumPhip, mSumPhim, corr, extrema);
     ctx->launches++;
     for (int j = 0; j < nLimiterIter; j++) {
-        mules_cell_lambda_kernel<<<(n + 127) / 128, 128, 0, st>>>(n, a->d_ownerStart, a->d_losortStart, a->d_losort, bs,
-                                                                  a->d_bCellFaces, lambda_d, lambdaB_d, phiCorr_d, phiCorrB_d,
+        mules_cell_lambda_kernel<<<(n + 127) / 128, 128, 0, st>>>(n, a->d_ownerStart.get(), a->d_losortStart.get(), a->d_losort.get(), bs,
+                                                                  a->d_bCellFaces.get(), lambda_d, lambdaB_d, phiCorr_d, phiCorrB_d,
                                                                   psiMaxn, psiMinn, sumPhip, mSumPhim, lambdam, lambdap);
-        mules_face_lambda_kernel<<<(nF + nB + 255) / 256, 256, 0, st>>>(nF, nB, nCoupledFaces, corr, a->d_l, a->d_u, a->d_bFaceCells, phiCorr_d,
+        mules_face_lambda_kernel<<<(nF + nB + 255) / 256, 256, 0, st>>>(nF, nB, nCoupledFaces, corr, a->d_l.get(), a->d_u.get(), a->d_bFaceCells.get(), phiCorr_d,
                                                                         phiCorrB_d, phiBDB_d, lambdam, lambdap, lambda_d,
                                                                         lambdaB_d);
         ctx->launches += 2;

@@ -256,7 +256,7 @@ int solve_pcg_fused(Solve &S, int pk)
     double *psi = S.psi, *b = S.src;
     double *pb[2] = {S.vec(0), S.vec(4)}, *w = S.vec(1), *rb[2] = {S.vec(2), S.vec(3)}, *z = S.vec(5);
     if (!pb[0] || !pb[1] || !w || !rb[0] || !rb[1] || !z) return B200LDU_ECUDA;
-    const double *rD = m->d_rD;
+    const double *rD = m->d_rD.get();
     const P2PRed pr = (S.ctx->nRanks > 1 && S.ctx->p2p) ? comm_p2p_red(S.ctx) : P2PRed();
     // the two sweeps leave their partials in separate buffers: a deferred step reads one while the sweep that
     // runs it writes the other
@@ -281,7 +281,7 @@ int solve_pcg_fused(Solve &S, int pk)
             PcgAinvOp<PreA> op;
             op.stop = stop;
             op.partials = partA;
-            op.rOld = rOld, op.rNew = rNew, op.w = w, op.p = pPrev, op.psi = psi, op.z = z, op.rD = m->d_rD;
+            op.rOld = rOld, op.rNew = rNew, op.w = w, op.p = pPrev, op.psi = psi, op.z = z, op.rD = m->d_rD.get();
             op.sc = sc;
             op.pre = preA;
             TRY(engine_launch_m(m, false, op));
@@ -314,7 +314,7 @@ int solve_pcg_fused(Solve &S, int pk)
         op.stop = stop;
         op.partials = partB;
         op.waitHalo = wait;
-        op.z = z, op.pOld = pPrev, op.pNew = pNew, op.out = w, op.diag = m->d_diag;
+        op.z = z, op.pOld = pPrev, op.pNew = pNew, op.out = w, op.diag = m->d_diag.get();
         op.sc = sc;
         op.pre = preB;
         TRY(engine_launch_m(m, false, op));
@@ -553,7 +553,7 @@ int solve_smooth(Solve &S)
 // diagonalSolver.C:62-81
 int solve_diagonal(Solve &S)
 {
-    const double *d = S.m->d_diag;
+    const double *d = S.m->d_diag.get();
     double *psi = S.psi;
     const double *b = S.src;
     return ew_launch<0>(S.ctx, S.m->a->L.nPad / 2, nullptr, nullptr, nullptr, [=] __device__(int i, double *) {
@@ -567,14 +567,7 @@ int gamg_run_cycles(Solve &S, long long maxBodies, int (*body)(void *), void *ar
     return run_iterations(S, maxBodies, [&](long long) -> int { return body(arg); });
 }
 
-double *Solve::vec(int k)
-{
-    while ((int)m->work.size() <= k) m->work.push_back(nullptr);
-    if (!m->work[k]) {
-        if (addr_alloc_vec(m->a, &m->work[k]) != B200LDU_OK) return nullptr;
-    }
-    return m->work[k];
-}
+double *Solve::vec(int k) { return addr_reuse_vec(m->a, m->work[k]); }
 
 int gamg_solve(Solve &S, b200ldu_gamg *g, const char *smoother); // gamg.cu
 
@@ -588,8 +581,8 @@ int solve_banded(b200ldu_matrix *m, const char *solver, const char *pre, const b
     Solve S;
     S.m = m;
     S.ctx = ctx;
-    S.sc = (SolverScalars *)m->d_scal;
-    S.partials = m->d_partials;
+    S.sc = m->d_scal.get();
+    S.partials = m->d_partials.get();
     S.psi = psi_b;
     S.src = src_b;
     if (controls)
@@ -601,17 +594,12 @@ int solve_banded(b200ldu_matrix *m, const char *solver, const char *pre, const b
 
     // residual history buffer on the device
     if (histCap > 0 && hist_h) {
-        if (m->histCap < histCap) {
-            if (m->d_hist) cudaFree(m->d_hist);
-            m->d_hist = nullptr;
-            CUDA_TRY(cudaMalloc((void **)&m->d_hist, sizeof(double) * (size_t)histCap));
-            m->histCap = histCap;
-        }
-        S.hist = m->d_hist;
+        TRY(m->d_hist.grow((size_t)histCap));
+        S.hist = m->d_hist.get();
     }
     // pinned flags + events
-    void *pin = nullptr;
-    TRY(ctx_pinned(ctx, 4096, &pin));
+    TRY(ctx->pinned.grow(4096));
+    char *pin = ctx->pinned.get();
     // a solve nested in another one (GAMG coarsest level) polls its own pair of flags
     static thread_local int depth = 0;
     struct Depth {
@@ -625,6 +613,14 @@ int solve_banded(b200ldu_matrix *m, const char *solver, const char *pre, const b
     }
     S.pinnedFlags = (int *)pin + 2 * (depth - 1);
     S.pinnedFlags[0] = S.pinnedFlags[1] = 0;
+    struct Events { // destroyed on every way out
+        cudaEvent_t *ev;
+        ~Events()
+        {
+            for (int i = 0; i < 2; i++)
+                if (ev[i]) cudaEventDestroy(ev[i]);
+        }
+    } events{S.ev};
     CUDA_TRY(cudaEventCreateWithFlags(&S.ev[0], cudaEventDisableTiming));
     CUDA_TRY(cudaEventCreateWithFlags(&S.ev[1], cudaEventDisableTiming));
 
@@ -747,12 +743,12 @@ int solve_banded(b200ldu_matrix *m, const char *solver, const char *pre, const b
     }
     if (rc == B200LDU_OK) {
         // read back the scalars (one synchronisation per solve)
-        SolverScalars *hp = (SolverScalars *)((char *)pin + 1024);
+        SolverScalars *hp = (SolverScalars *)(pin + 1024);
         CUDA_TRY(cudaMemcpyAsync(hp, S.sc, sizeof(SolverScalars), cudaMemcpyDeviceToHost, ctx->stream));
-        unsigned long long *peerErr = (unsigned long long *)((char *)pin + 2048);
+        unsigned long long *peerErr = (unsigned long long *)(pin + 2048);
         *peerErr = 0;
-        if (ctx->d_seq) // a bounded wait on a peer's flag gave up (engine.cuh spin_until)
-            CUDA_TRY(cudaMemcpyAsync(peerErr, ctx->d_seq + 7, sizeof(*peerErr), cudaMemcpyDeviceToHost, ctx->stream));
+        if (ctx->d_seq.get()) // a bounded wait on a peer's flag gave up (engine.cuh spin_until)
+            CUDA_TRY(cudaMemcpyAsync(peerErr, ctx->d_seq.get() + 7, sizeof(*peerErr), cudaMemcpyDeviceToHost, ctx->stream));
         CUDA_TRY(cudaStreamSynchronize(ctx->stream));
         if (*peerErr) {
             b200_set_error("solve: timed out waiting for a peer GPU's halo / all-reduce flag (a rank died or did not "
@@ -779,14 +775,12 @@ int solve_banded(b200ldu_matrix *m, const char *solver, const char *pre, const b
             if (!strcmp(perf->solverName, "smoothSolver") && S.c.nSweeps > 0) k = perf->nIterations / S.c.nSweeps + 1;
             if (k > histCap) k = histCap;
             if (S.noScalars || S.fixedSweeps) k = 0;
-            if (k > 0) CUDA_TRY(cudaMemcpy(hist_h, m->d_hist, sizeof(double) * (size_t)k, cudaMemcpyDeviceToHost));
+            if (k > 0) CUDA_TRY(cudaMemcpy(hist_h, m->d_hist.get(), sizeof(double) * (size_t)k, cudaMemcpyDeviceToHost));
             for (int i = k; i < histCap; i++) hist_h[i] = NAN;
         }
     } else {
         cudaStreamSynchronize(ctx->stream);
     }
-    cudaEventDestroy(S.ev[0]);
-    cudaEventDestroy(S.ev[1]);
     return rc;
 }
 
@@ -800,10 +794,8 @@ extern "C" int b200ldu_solve(b200ldu_matrix *m, const char *solver, const char *
     }
     CUDA_TRY(cudaSetDevice(m->a->ctx->device));
     b200ldu_addr *a = m->a;
-    // banded copies of psi and source live with the matrix workspace (slots 14, 15)
-    Solve tmp;
-    tmp.m = m;
-    double *psi_b = tmp.vec(14), *src_b = tmp.vec(15);
+    // banded copies of psi and source live with the matrix workspace
+    double *psi_b = addr_reuse_vec(a, m->work[WORK_PSI_B]), *src_b = addr_reuse_vec(a, m->work[WORK_SRC_B]);
     if (!psi_b || !src_b) return B200LDU_ECUDA;
     TRY(to_banded(a, psi_d, psi_b));
     TRY(to_banded(a, source_d, src_b));
@@ -826,9 +818,7 @@ extern "C" int b200ldu_solve_host(b200ldu_matrix *m, const char *solver, const c
     b200ldu_ctx *ctx = a->ctx;
     CUDA_TRY(cudaSetDevice(ctx->device));
     size_t bytes = sizeof(double) * (size_t)a->nCells;
-    Solve tmp;
-    tmp.m = m;
-    double *psi_d = tmp.vec(12), *src_d = tmp.vec(13);
+    double *psi_d = addr_reuse_vec(a, m->work[WORK_HOST_PSI]), *src_d = addr_reuse_vec(a, m->work[WORK_HOST_SRC]);
     if (!psi_d || !src_d) return B200LDU_ECUDA;
     // host buffers may be pageable: cudaMemcpyAsync then stages through the driver's pinned pool
     CUDA_TRY(cudaMemcpyAsync(psi_d, psi_h, bytes, cudaMemcpyHostToDevice, ctx->stream));

@@ -21,7 +21,7 @@ struct Solve {
     bool noScalars = false;
     bool useGraph = false; // replay iteration chunks as a CUDA graph
     int gamgFinestSweeps = 0; // GAMG: finest-level sweeps per cycle (result-buffer parity)
-    double *vec(int k); // workspace vector k of the matrix (allocated once, reused)
+    double *vec(int k); // workspace vector k < WORK_SOLVER_SLOTS of the matrix (allocated once, reused)
 };
 
 int solve_banded(b200ldu_matrix *m, const char *solver, const char *pre, const b200ldu_controls *controls,
